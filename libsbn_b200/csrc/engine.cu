@@ -38,7 +38,7 @@ thread_local std::string g_last_error;
 // one category each, so powers of two); other counts run padded
 // with zero-weight categories.
 int PadCategories(int c) {
-  for (int supported : {1, 2, 4, 8, 16})
+  for (int supported : {1, 2, 4, 8, 16, 32})
     if (c <= supported) return supported;
   return 0;
 }
@@ -314,6 +314,9 @@ LaunchPlan Dispatch(sbnb_engine* e, const OeParams& p, bool grad, bool rescale, 
       return DispatchModesOe<8, 2, 2>(e, p, grad, rescale, launch, chunks_override);
     case 16:
       return DispatchModesOe<16, 2, 2>(e, p, grad, rescale, launch, chunks_override);
+    case 32:
+      // (one pattern column per warp: tiles of 4 warps x 4 patterns)
+      return DispatchModesOe<32, 4, 4>(e, p, grad, rescale, launch, chunks_override);
   }
   Fail(SBNB_ERR_INVALID_ARGUMENT, "Unsupported category count.");
 }
@@ -1072,7 +1075,7 @@ std::unique_ptr<sbnb_engine> CreateEngine(const char* substitution, const char* 
   engine->categories = engine->spec.category_count;
   engine->padded_categories = PadCategories(engine->categories);
   Require(engine->padded_categories > 0,
-          "At most 16 rate categories are supported by the fused tree walk (libhmsbeagle_b200.so, the "
+          "At most 32 rate categories are supported by the fused tree walk (libhmsbeagle_b200.so, the "
           "BEAGLE-compatible device library behind the unmodified FatBeagle, takes any number).");
   SBNB_CUDA(cudaStreamCreateWithFlags(&engine->stream, cudaStreamNonBlocking));
   SBNB_CUDA(cudaEventCreateWithFlags(&engine->staging_free, cudaEventDisableTiming));

@@ -97,8 +97,11 @@ struct WalkParams {
 };
 
 // Shared memory of one CTA (host and device agree through these).
-// Per-item model constants: Q[16], p_c[16], p_c r_c[16], p_c dr_c/dshape[16], pi[4].
-constexpr int kModelSmemDoubles = 16 + 3 * kMaxCategories + 4;
+// Per-item model constants of a walk over C (padded) categories: Q[16], then p_c, r_c and
+// dr_c/dshape with ModelSmemCategories(C) entries each, pi[4].  Up to 16 categories the
+// arrays keep 16 entries.
+__host__ __device__ constexpr int ModelSmemCategories(int C) { return C > 16 ? C : 16; }
+__host__ __device__ constexpr int ModelSmemDoubles(int C) { return 16 + 3 * ModelSmemCategories(C) + 4; }
 
 // ---------------------------------------------------------------------------
 // mbarrier / TMA bulk-copy helpers (PTX; see blackwell_cuda_programming.md)

@@ -26,6 +26,15 @@ void AppendBlock(ModelSpec* spec, const std::string& entire_key,
   spec->blocks[entire_key] = {start, spec->param_count - start};
 }
 
+// One lane of a warp per rate category in the fused tree walk: 1 to 32.
+void CheckCategoryCount(const ModelSpec& spec, const std::string& site) {
+  if (spec.category_count < 1 || spec.category_count > kMaxCategories)
+    Fail(SBNB_ERR_INVALID_ARGUMENT,
+         "Site model category count out of range [1," + std::to_string(kMaxCategories) + "]: " + site +
+             " (the fused tree walk gives each rate category one lane of a warp; libhmsbeagle_b200.so, the "
+             "BEAGLE-compatible device library behind the unmodified FatBeagle, takes any number)");
+}
+
 }  // namespace
 
 ModelSpec ModelSpec::Parse(const std::string& substitution, const std::string& site,
@@ -60,9 +69,7 @@ ModelSpec ModelSpec::Parse(const std::string& substitution, const std::string& s
         Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);
       }
     }
-    if (spec.category_count < 1 || spec.category_count > kMaxCategories)
-      Fail(SBNB_ERR_INVALID_ARGUMENT,
-           "Site model category count out of range [1,16]: " + site);
+    CheckCategoryCount(spec, site);
     AppendBlock(&spec, "entire site", {{"Weibull shape", 1}});
   } else if (site.rfind("gamma", 0) == 0) {
     // Not in the reference (its "Gamma-4" is weibull+4): "gamma" (4 categories) or "gamma+K".
@@ -78,9 +85,7 @@ ModelSpec ModelSpec::Parse(const std::string& substitution, const std::string& s
     } else if (site != "gamma") {
       Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);
     }
-    if (spec.category_count < 1 || spec.category_count > kMaxCategories)
-      Fail(SBNB_ERR_INVALID_ARGUMENT,
-           "Site model category count out of range [1,16]: " + site);
+    CheckCategoryCount(spec, site);
     AppendBlock(&spec, "entire site", {{"Gamma shape", 1}});
   } else {
     Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);

@@ -34,6 +34,10 @@ struct ModelSpec {
   int SubstitutionGradientSize() const;
 };
 
+// The fused tree walk gives every rate category of a site pattern its own lane, so a
+// pattern takes at most one warp of categories.
+constexpr int kMaxCategories = 32;
+
 // Everything the kernels need to know about the substitution + site model of
 // one (virtual) tree.  Row-major 4x4 blocks, as BEAGLE receives them
 // (fat_beagle.cpp:289-293).
@@ -43,12 +47,10 @@ struct ModelTables {
   double eval[4];       // Lambda
   double freqs[4];      // pi
   double q[16];         // rate matrix Q (unit expected rate)
-  double rates[16];     // category rates r_c           (first category_count used)
-  double weights[16];   // category proportions p_c
-  double drates[16];    // d r_c / d shape (Weibull, Gamma; 0 for a constant site model)
+  double rates[kMaxCategories];     // category rates r_c           (first category_count used)
+  double weights[kMaxCategories];   // category proportions p_c
+  double drates[kMaxCategories];    // d r_c / d shape (Weibull, Gamma; 0 for a constant site model)
 };
-
-constexpr int kMaxCategories = 16;
 
 // substitution_model.cpp:17-80 (GTR), substitution_model.hpp:59-74 (JC69).
 // `params` points at the "entire substitution" block of a row.

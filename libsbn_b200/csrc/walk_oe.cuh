@@ -423,8 +423,19 @@ __global__ void PeerSumKernel(double* __restrict__ out, PeerPointers peers, int3
 #ifndef SBNB_OE_PREFETCH
 #define SBNB_OE_PREFETCH (SBNB_OE_STAGES / 2)
 #endif
-__host__ __device__ constexpr int OeStages(int C) { return C >= 8 ? 4 : SBNB_OE_STAGES; }  // operand ring depth
-__host__ __device__ constexpr int OePrefetchOps(int C) { return C >= 8 ? 2 : SBNB_OE_PREFETCH; }
+// At 32 categories one op's operands take ~25 KB (37 KB with the analytic substitution
+// gradient), so the ring is shallow and requests run one op ahead.  An op's request waits
+// until every warp has left the op kStages - kPrefetch places before it: with a margin of one
+// op (2 stages) the first warp waits for the last at every op, which costs the gradient walk
+// 3.6x (measured); the logL-only walk, with no pre-order half, loses less to that than it
+// would to going from three resident CTAs per SM to two.
+#ifndef SBNB_OE_STAGES_32
+#define SBNB_OE_STAGES_32 3  // gradient walks at 32 categories
+#endif
+__host__ __device__ constexpr int OeStages(int C, bool grad) {  // operand ring depth
+  return C >= 32 ? (grad ? SBNB_OE_STAGES_32 : 2) : C >= 8 ? 4 : SBNB_OE_STAGES;
+}
+__host__ __device__ constexpr int OePrefetchOps(int C) { return C >= 32 ? 1 : C >= 8 ? 2 : SBNB_OE_PREFETCH; }
 __host__ __device__ constexpr int OeGroup(int C) { return kThreads / C; }  // patterns per j-slab
 __host__ __device__ constexpr int OeTilePatterns(int C, int K) { return OeGroup(C) * K; }
 __host__ __device__ constexpr int OeTipBytes(int C, int K) { return (OeTilePatterns(C, K) + 15) / 16 * 16; }
@@ -438,8 +449,8 @@ __host__ __device__ constexpr int OeReadbackBytes(int K) { return 2 * K * 2 * kT
 // model constants of the analytic substitution gradient: V, V^-1, and V^-1 e_s per tip state
 constexpr int kOeSubstSmemDoubles = 16 + 16 + 20;
 __host__ __device__ constexpr size_t OeSmemBytes(int C, int K, bool grad, bool subst = false) {
-  return static_cast<size_t>(OeStages(C)) * OeStageBytes(C, K, subst) + 2 * OeStages(C) * 8 +
-         (kModelSmemDoubles + kOeSubstSmemDoubles) * 8 + 16 + 2 * kWarps * 8 + (grad ? OeReadbackBytes(K) : 0);
+  return static_cast<size_t>(OeStages(C, grad)) * OeStageBytes(C, K, subst) + 2 * OeStages(C, grad) * 8 +
+         (ModelSmemDoubles(C) + kOeSubstSmemDoubles) * 8 + 16 + 2 * kWarps * 8 + (grad ? OeReadbackBytes(K) : 0);
 }
 // Resident CTAs per SM the register allocation is held to.
 __host__ __device__ constexpr int OeMinBlocks(int K, bool grad, bool subst = false) {
@@ -532,7 +543,7 @@ __device__ __forceinline__ void NormalizeOe(double (&v)[K][4], int (&exps)[K]) {
 template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false>
 __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWalkOeKernel(const OeParams p) {
   static_assert(GRAD || !SUBST, "the substitution gradient rides on the pre-order pass");
-  static_assert((C & (C - 1)) == 0 && C >= 1 && C <= 16, "lanes per pattern must be a power of two");
+  static_assert((C & (C - 1)) == 0 && C >= 1 && C <= 32, "lanes per pattern must be a power of two");
   static_assert(OeTilePatterns(C, K) % 16 == 0, "tiles must start on 16-byte boundaries of the tip rows");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int tid = threadIdx.x;
@@ -547,7 +558,7 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
   const int internal_count = n - 1;
   const int node_count = 2 * n - 1;
   const int ops_total = GRAD ? 2 * internal_count : internal_count;
-  constexpr int kStages = OeStages(C);
+  constexpr int kStages = OeStages(C, GRAD);
   constexpr int kPrefetch = OePrefetchOps(C);
   constexpr int kTilePatterns = OeTilePatterns(C, K);
   constexpr int kTipBytes = OeTipBytes(C, K);
@@ -567,9 +578,9 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
   uint64_t* const empty = full + kStages;
   double* const q_smem = reinterpret_cast<double*>(empty + kStages);
   double* const cat_weight_smem = q_smem + 16;
-  double* const rate_weight_smem = cat_weight_smem + kMaxCategories;
-  double* const drate_weight_smem = rate_weight_smem + kMaxCategories;
-  double* const freqs_smem = drate_weight_smem + kMaxCategories;
+  double* const rate_weight_smem = cat_weight_smem + ModelSmemCategories(C);
+  double* const drate_weight_smem = rate_weight_smem + ModelSmemCategories(C);
+  double* const freqs_smem = drate_weight_smem + ModelSmemCategories(C);
   double* const evec_smem = freqs_smem + 4;  // V, V^-1 and V^-1 e_s (s = A C G T, gap): analytic substitution gradient
   double* const ivec_smem = evec_smem + 16;
   double* const tip_z_smem = ivec_smem + 16;
@@ -624,6 +635,11 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
         evec_smem[tid] = model.evec[tid];
         ivec_smem[tid] = model.ivec[tid];
       }
+    }
+    if (C > 16 && tid >= 16 && tid < C) {
+      cat_weight_smem[tid] = model.weights[tid];
+      rate_weight_smem[tid] = model.rates[tid];
+      drate_weight_smem[tid] = model.drates[tid];
     }
     if (SUBST && tid >= 32 && tid < 52) {
       // V^-1 L for a tip: column s of V^-1 for a resolved state, the row sums for a gap
