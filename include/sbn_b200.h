@@ -72,6 +72,26 @@ int sbnb_engine_create(const char* substitution, const char* site, const char* c
 void sbnb_engine_destroy(sbnb_engine* engine);
 
 /*
+ * How the bytes of an alignment ([taxon][pattern]) encode its tips.
+ *   SBNB_TIPS_STATES            0..3 = A,C,G,T, anything >= 4 = gap/unknown (the
+ *                               reference's symbol table: degenerate nucleotides are gaps).
+ *   SBNB_TIPS_NUCLEOTIDE_MASKS  the set of states a character allows: bit 0 = A, bit 1 = C,
+ *                               bit 2 = G, bit 3 = T; 15 = missing (N X ? -), R = A|G = 5 and
+ *                               so on.  A tip then enters the likelihood as the partial
+ *                               vector of its bits (BEAGLE's tip partials).  0 and values
+ *                               above 15 are refused with SBNB_ERR_INVALID_ARGUMENT.
+ * An alignment of masks without a two- or three-state mask gives results bitwise identical
+ * to the same alignment as states.
+ */
+enum { SBNB_TIPS_STATES = 0, SBNB_TIPS_NUCLEOTIDE_MASKS = 1 };
+/* sbnb_engine_create with the tips in the given encoding (sbnb_engine_create is the
+ * SBNB_TIPS_STATES case). */
+int sbnb_engine_create_encoded(const char* substitution, const char* site, const char* clock,
+                               int32_t taxon_count, int64_t pattern_count, const uint8_t* tips,
+                               int32_t tip_encoding, const double* pattern_weights, int32_t device,
+                               sbnb_engine** out);
+
+/*
  * A device group: one engine over several GPUs of the box, replacing the
  * reference's thread_count FatBeagle instances and the thread pool that fans a
  * collection over them (engine.cpp:17-27, fat_beagle.hpp:119-149) -- one host thread
@@ -91,6 +111,12 @@ int sbnb_engine_create_multi(const char* substitution, const char* site, const c
                              int32_t taxon_count, int64_t pattern_count, const uint8_t* tip_states,
                              const double* pattern_weights, const int32_t* devices,
                              int32_t device_count, int32_t shard_axis, sbnb_engine** out);
+/* sbnb_engine_create_multi with the tips in the given encoding (see sbnb_engine_create_encoded). */
+int sbnb_engine_create_multi_encoded(const char* substitution, const char* site, const char* clock,
+                                     int32_t taxon_count, int64_t pattern_count, const uint8_t* tips,
+                                     int32_t tip_encoding, const double* pattern_weights,
+                                     const int32_t* devices, int32_t device_count, int32_t shard_axis,
+                                     sbnb_engine** out);
 /*
  * How the "substitution_model" block of a gradient call (GTR: 8 entries, HKY: 4) is
  * computed.  The reference takes central differences of 16 full log-likelihood

@@ -68,6 +68,15 @@ int sbnb_gp_create(int32_t taxon_count, int64_t pattern_count, const uint8_t* ti
                    int32_t gpcsp_count, double rescaling_threshold, const double* sbn_prior,
                    const double* unconditional_node_probabilities, int32_t node_count,
                    const double* inverted_sbn_prior, int32_t device, sbnb_gp_engine** out);
+/* sbnb_gp_create with the tips in the given encoding (SBNB_TIPS_*, sbn_b200.h;
+ * sbnb_gp_create is the SBNB_TIPS_STATES case).  With SBNB_TIPS_NUCLEOTIDE_MASKS a leaf
+ * PLV entry is bit s of the tip's mask, in every category; 15 is the all-ones gap. */
+int sbnb_gp_create_encoded(int32_t taxon_count, int64_t pattern_count, const uint8_t* tips,
+                           int32_t tip_encoding, const double* pattern_weights, int64_t site_count,
+                           int32_t plv_count, int32_t gpcsp_count, double rescaling_threshold,
+                           const double* sbn_prior, const double* unconditional_node_probabilities,
+                           int32_t node_count, const double* inverted_sbn_prior, int32_t device,
+                           sbnb_gp_engine** out);
 void sbnb_gp_destroy(sbnb_gp_engine* engine);
 
 /*

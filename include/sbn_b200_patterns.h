@@ -48,6 +48,17 @@ extern "C" {
 int sbnb_compress_site_patterns(int32_t taxon_count, int64_t site_count, const char* sequences,
                                 int32_t device, uint8_t* out_patterns, double* out_weights,
                                 int64_t* out_pattern_count, double* out_device_ms);
+/*
+ * sbnb_compress_site_patterns with the output in the given tip encoding (SBNB_TIPS_*,
+ * sbn_b200.h; sbnb_compress_site_patterns is the SBNB_TIPS_STATES case).  With
+ * SBNB_TIPS_NUCLEOTIDE_MASKS the characters map through the IUPAC table, upper and lower
+ * case: A C G T = 1 2 4 8, U = T, R Y S W K M B D H V = the masks of the states they allow,
+ * N X ? - = 15; columns that differ only in degenerate codes are different patterns.
+ */
+int sbnb_compress_site_patterns_encoded(int32_t taxon_count, int64_t site_count, const char* sequences,
+                                        int32_t tip_encoding, int32_t device, uint8_t* out_patterns,
+                                        double* out_weights, int64_t* out_pattern_count,
+                                        double* out_device_ms);
 
 #ifdef __cplusplus
 }

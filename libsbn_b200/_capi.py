@@ -51,6 +51,9 @@ _c = ctypes
 SIGNATURES = {
     "sbnb_compress_site_patterns": (_c.c_int, [_c.c_int32, _c.c_int64, _c.c_char_p, _c.c_int32, _P(_c.c_uint8),
                                                _P(_c.c_double), _P(_c.c_int64), _P(_c.c_double)]),
+    "sbnb_compress_site_patterns_encoded": (_c.c_int, [_c.c_int32, _c.c_int64, _c.c_char_p, _c.c_int32, _c.c_int32,
+                                                       _P(_c.c_uint8), _P(_c.c_double), _P(_c.c_int64),
+                                                       _P(_c.c_double)]),
     "sbnb_last_error": (_c.c_char_p, []),
     "sbnb_device_count": (_c.c_int, []),
     "sbnb_engine_create": (_c.c_int, [_c.c_char_p, _c.c_char_p, _c.c_char_p, _c.c_int32, _c.c_int64,
@@ -58,6 +61,12 @@ SIGNATURES = {
     "sbnb_engine_create_multi": (_c.c_int, [_c.c_char_p, _c.c_char_p, _c.c_char_p, _c.c_int32, _c.c_int64,
                                             _P(_c.c_uint8), _P(_c.c_double), _P(_c.c_int32), _c.c_int32,
                                             _c.c_int32, _P(_c.c_void_p)]),
+    "sbnb_engine_create_encoded": (_c.c_int, [_c.c_char_p, _c.c_char_p, _c.c_char_p, _c.c_int32, _c.c_int64,
+                                              _P(_c.c_uint8), _c.c_int32, _P(_c.c_double), _c.c_int32,
+                                              _P(_c.c_void_p)]),
+    "sbnb_engine_create_multi_encoded": (_c.c_int, [_c.c_char_p, _c.c_char_p, _c.c_char_p, _c.c_int32, _c.c_int64,
+                                                    _P(_c.c_uint8), _c.c_int32, _P(_c.c_double), _P(_c.c_int32),
+                                                    _c.c_int32, _c.c_int32, _P(_c.c_void_p)]),
     "sbnb_engine_device_count": (_c.c_int32, [_c.c_void_p]),
     "sbnb_engine_set_substitution_gradient": (_c.c_int, [_c.c_void_p, _c.c_int32]),
     "sbnb_engine_destroy": (None, [_c.c_void_p]),
@@ -111,6 +120,10 @@ SIGNATURES.update({
     "sbnb_gp_create": (_c.c_int, [_c.c_int32, _c.c_int64, _P(_c.c_uint8), _P(_c.c_double), _c.c_int64, _c.c_int32,
                                   _c.c_int32, _c.c_double, _P(_c.c_double), _P(_c.c_double), _c.c_int32,
                                   _P(_c.c_double), _c.c_int32, _P(_c.c_void_p)]),
+    "sbnb_gp_create_encoded": (_c.c_int, [_c.c_int32, _c.c_int64, _P(_c.c_uint8), _c.c_int32, _P(_c.c_double),
+                                          _c.c_int64, _c.c_int32, _c.c_int32, _c.c_double, _P(_c.c_double),
+                                          _P(_c.c_double), _c.c_int32, _P(_c.c_double), _c.c_int32,
+                                          _P(_c.c_void_p)]),
     "sbnb_gp_destroy": (None, [_c.c_void_p]),
     "sbnb_gp_process_operations": (_c.c_int, [_c.c_void_p, _P(_c.c_int32), _c.c_int64]),
     "sbnb_gp_set_substitution_model": (_c.c_int, [_c.c_void_p, _c.c_char_p, _P(_c.c_double), _c.c_int32]),
@@ -148,6 +161,9 @@ STAGE_SUBSTITUTION_FD = 2
 STAGE_SUBSTITUTION_ANALYTIC = 4
 SUBSTITUTION_SUMS = 20
 SHARD_TREES = 0
+TIPS_STATES = 0
+TIPS_NUCLEOTIDE_MASKS = 1
+TIP_ENCODINGS = {"states": TIPS_STATES, "masks": TIPS_NUCLEOTIDE_MASKS}
 SHARD_PATTERNS = 1
 SUBSTITUTION_ANALYTIC = 0
 SUBSTITUTION_FINITE_DIFFERENCES = 1
@@ -185,6 +201,13 @@ def as_double_ptr(array):
         return None
     assert array.dtype == np.float64 and array.flags["C_CONTIGUOUS"]
     return array.ctypes.data_as(_P(_c.c_double))
+
+
+def tip_encoding(name):
+    """'states' (0..3 = ACGT, >= 4 gap) or 'masks' (nucleotide masks 1..15) -> SBNB_TIPS_*."""
+    if name not in TIP_ENCODINGS:
+        raise RuntimeError("tip_encoding must be 'states' or 'masks'.")
+    return TIP_ENCODINGS[name]
 
 
 def as_int32_ptr(array):

@@ -34,8 +34,16 @@ class Beagle:
         a = np.ascontiguousarray(a, dtype=np.int32)
         return a, a.ctypes.data_as(_I)
 
-    def set_tips(self, states, weights, use_tip_states):
+    def set_tips(self, states, weights, use_tip_states, masks=False):
+        """Tip states (use_tip_states) or tip partials built from them; masks=True: `states`
+        are nucleotide masks, and each tip's partial is the indicator vector of its bits."""
         for tip in range(self.n):
+            if masks:
+                bits = np.asarray(states[tip], dtype=np.int64)
+                partial = np.ascontiguousarray(((bits[:, None] >> np.arange(4)) & 1).astype(np.float64))
+                keep, ptr = self._d(partial)
+                self.ok(self.lib.beagleSetTipPartials(self.handle, tip, ptr))
+                continue
             if use_tip_states:
                 keep, ptr = self._i(states[tip])
                 self.ok(self.lib.beagleSetTipStates(self.handle, tip, ptr))

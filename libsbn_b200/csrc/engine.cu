@@ -62,7 +62,8 @@ struct sbnb_engine {
   int categories = 1;         // C
   int padded_categories = 1;  // instantiated count >= C (extra categories have weight 0)
   // host copy of the alignment (shared by the children of a device group)
-  std::shared_ptr<const std::vector<uint8_t>> host_tips;    // [taxon][pattern], states clamped to 0..4
+  std::shared_ptr<const std::vector<uint8_t>> host_tips;    // [taxon][pattern], tip codes 0..14 (walk_oe.cuh)
+  bool ambiguous = false;  // some tip code is >= kFirstAmbiguousCode: the walks sum tip-table rows
   std::shared_ptr<const std::vector<double>> host_weights;  // [pattern]
   cudaStream_t stream = nullptr;
   // CUDA-event pairs bracketing the base tree-walk launch of the last
@@ -213,12 +214,12 @@ struct LaunchPlan {
 };
 
 // Plans (and launches) TreeWalkOeKernel, whose tiles are kThreads / C * K patterns.
-template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false>
+template <int C, int K, bool GRAD, bool RESCALE, bool SUBST, bool AMBIG>
 LaunchPlan PlanAndLaunchOe(sbnb_engine* e, OeParams p, bool launch, int chunks_override) {
-  auto kernel = TreeWalkOeKernel<C, K, GRAD, RESCALE, SUBST>;
+  auto kernel = TreeWalkOeKernel<C, K, GRAD, RESCALE, SUBST, AMBIG>;
   // (SBNB_EXTRA_SMEM: development aid -- pads the request to lower the resident CTA count)
   const size_t smem =
-      OeSmemBytes(C, K, GRAD, SUBST) + static_cast<size_t>(std::max(0, EnvInt("SBNB_EXTRA_SMEM", 0)));
+      OeSmemBytes(C, K, GRAD, SUBST, AMBIG) + static_cast<size_t>(std::max(0, EnvInt("SBNB_EXTRA_SMEM", 0)));
   // (attributes and occupancy of a kernel are asked for once per engine)
   auto known = e->occupancy.find(reinterpret_cast<const void*>(kernel));
   if (known == e->occupancy.end() || known->second.first != smem) {
@@ -279,21 +280,30 @@ LaunchPlan PlanAndLaunchOe(sbnb_engine* e, OeParams p, bool launch, int chunks_o
   return plan;
 }
 
-template <int C, int K, bool GRAD, bool SUBST = false>
+template <int C, int K, bool GRAD, bool SUBST, bool AMBIG>
 LaunchPlan DispatchRescale(sbnb_engine* e, const OeParams& p, bool rescale, bool launch, int chunks_override) {
-  return rescale ? PlanAndLaunchOe<C, K, GRAD, true, SUBST>(e, p, launch, chunks_override)
-                 : PlanAndLaunchOe<C, K, GRAD, false, SUBST>(e, p, launch, chunks_override);
+  return rescale ? PlanAndLaunchOe<C, K, GRAD, true, SUBST, AMBIG>(e, p, launch, chunks_override)
+                 : PlanAndLaunchOe<C, K, GRAD, false, SUBST, AMBIG>(e, p, launch, chunks_override);
 }
 
 // K_GRAD / K_LOGL patterns per thread for the gradient / logL-only walk; a gradient walk
 // with p.subst_partial set also accumulates the analytic substitution-gradient sums.
-template <int C, int K_GRAD, int K_LOGL>
+template <int C, int K_GRAD, int K_LOGL, bool AMBIG>
 LaunchPlan DispatchModesOe(sbnb_engine* e, const OeParams& p, bool grad, bool rescale, bool launch,
                            int chunks_override) {
   if (grad && p.subst_partial != nullptr)
-    return DispatchRescale<C, K_GRAD, true, true>(e, p, rescale, launch, chunks_override);
-  return grad ? DispatchRescale<C, K_GRAD, true>(e, p, rescale, launch, chunks_override)
-              : DispatchRescale<C, K_LOGL, false>(e, p, rescale, launch, chunks_override);
+    return DispatchRescale<C, K_GRAD, true, true, AMBIG>(e, p, rescale, launch, chunks_override);
+  return grad ? DispatchRescale<C, K_GRAD, true, false, AMBIG>(e, p, rescale, launch, chunks_override)
+              : DispatchRescale<C, K_LOGL, false, false, AMBIG>(e, p, rescale, launch, chunks_override);
+}
+
+// An alignment with ambiguous tip codes runs the walks that sum tip-table rows; any other
+// runs the walks that read one row per tip.
+template <int C, int K_GRAD, int K_LOGL>
+LaunchPlan DispatchTipsOe(sbnb_engine* e, const OeParams& p, bool grad, bool rescale, bool launch,
+                          int chunks_override) {
+  return e->ambiguous ? DispatchModesOe<C, K_GRAD, K_LOGL, true>(e, p, grad, rescale, launch, chunks_override)
+                      : DispatchModesOe<C, K_GRAD, K_LOGL, false>(e, p, grad, rescale, launch, chunks_override);
 }
 
 // Patterns per thread K: more of them amortise the per-op overhead (operand requests,
@@ -304,19 +314,19 @@ LaunchPlan Dispatch(sbnb_engine* e, const OeParams& p, bool grad, bool rescale, 
                     int chunks_override) {
   switch (e->padded_categories) {
     case 1:
-      return DispatchModesOe<1, 2, 4>(e, p, grad, rescale, launch, chunks_override);
+      return DispatchTipsOe<1, 2, 4>(e, p, grad, rescale, launch, chunks_override);
     case 2:
-      return DispatchModesOe<2, 2, 4>(e, p, grad, rescale, launch, chunks_override);
+      return DispatchTipsOe<2, 2, 4>(e, p, grad, rescale, launch, chunks_override);
     case 4:
       // (measured: 4 patterns per thread at 12 warps/SM beat 2 at 16 warps/SM by 8 %)
-      return DispatchModesOe<4, 4, 4>(e, p, grad, rescale, launch, chunks_override);
+      return DispatchTipsOe<4, 4, 4>(e, p, grad, rescale, launch, chunks_override);
     case 8:
-      return DispatchModesOe<8, 2, 2>(e, p, grad, rescale, launch, chunks_override);
+      return DispatchTipsOe<8, 2, 2>(e, p, grad, rescale, launch, chunks_override);
     case 16:
-      return DispatchModesOe<16, 2, 2>(e, p, grad, rescale, launch, chunks_override);
+      return DispatchTipsOe<16, 2, 2>(e, p, grad, rescale, launch, chunks_override);
     case 32:
       // (one pattern column per warp: tiles of 4 warps x 4 patterns)
-      return DispatchModesOe<32, 4, 4>(e, p, grad, rescale, launch, chunks_override);
+      return DispatchTipsOe<32, 4, 4>(e, p, grad, rescale, launch, chunks_override);
   }
   Fail(SBNB_ERR_INVALID_ARGUMENT, "Unsupported category count.");
 }
@@ -1045,16 +1055,41 @@ RootedView ViewOf(const sbnb_tree_batch* trees, int t, int n) {
   return view;
 }
 
+// The tip codes of an alignment (walk_oe.cuh): states 0..3 stay, anything >= 4 is the gap
+// code 4; nucleotide masks become codes 0..14, and 0 or > 15 is refused.
+std::shared_ptr<const std::vector<uint8_t>> TipCodes(int32_t taxon_count, int64_t pattern_count,
+                                                     const uint8_t* tips, int32_t encoding, bool* ambiguous) {
+  auto codes = std::make_shared<std::vector<uint8_t>>(static_cast<size_t>(taxon_count) * pattern_count);
+  *ambiguous = false;
+  if (encoding == SBNB_TIPS_STATES) {
+    for (size_t i = 0; i < codes->size(); i++) (*codes)[i] = tips[i] < 4 ? tips[i] : 4;
+    return codes;
+  }
+  uint8_t code_of[16] = {};
+  for (int code = 0; code < kTipCodes; code++) code_of[TipCodeMask(code)] = static_cast<uint8_t>(code);
+  for (size_t i = 0; i < codes->size(); i++) {
+    const uint8_t mask = tips[i];
+    if (mask == 0 || mask > 15)
+      Fail(SBNB_ERR_INVALID_ARGUMENT, "Invalid nucleotide mask " + std::to_string(mask) + " at taxon " +
+                                          std::to_string(i / pattern_count) + ", pattern " +
+                                          std::to_string(i % pattern_count) + " (masks are 1..15).");
+    (*codes)[i] = code_of[mask];
+    *ambiguous = *ambiguous || code_of[mask] >= kFirstAmbiguousCode;
+  }
+  return codes;
+}
+
 // Engine::Engine + FatBeagle::FatBeagle for one device.  `sibling` (a child of the same
 // device group) shares its host copy of the alignment.
 std::unique_ptr<sbnb_engine> CreateEngine(const char* substitution, const char* site, const char* clock,
-                                          int32_t taxon_count, int64_t pattern_count, const uint8_t* tip_states,
-                                          const double* pattern_weights, int32_t device,
+                                          int32_t taxon_count, int64_t pattern_count, const uint8_t* tips,
+                                          int32_t tip_encoding, const double* pattern_weights, int32_t device,
                                           const sbnb_engine* sibling) {
   Require(substitution && site && clock, "NULL model specification string.");
   Require(taxon_count >= 2, "Need at least 2 taxa.");
   Require(pattern_count >= 1, "Need at least 1 site pattern.");
-  Require(tip_states && pattern_weights, "NULL tip_states / pattern_weights.");
+  Require(tips && pattern_weights, "NULL tip_states / pattern_weights.");
+  Require(tip_encoding == SBNB_TIPS_STATES || tip_encoding == SBNB_TIPS_NUCLEOTIDE_MASKS, "Unknown tip encoding.");
   auto engine = std::make_unique<sbnb_engine>();
   engine->spec = ModelSpec::Parse(substitution, site, clock);
   int device_count = 0;
@@ -1085,11 +1120,10 @@ std::unique_ptr<sbnb_engine> CreateEngine(const char* substitution, const char* 
   }
   if (sibling) {
     engine->host_tips = sibling->host_tips;
+    engine->ambiguous = sibling->ambiguous;
     engine->host_weights = sibling->host_weights;
   } else {
-    auto tips = std::make_shared<std::vector<uint8_t>>(static_cast<size_t>(taxon_count) * pattern_count);
-    for (size_t i = 0; i < tips->size(); i++) (*tips)[i] = tip_states[i] < 4 ? tip_states[i] : 4;
-    engine->host_tips = tips;
+    engine->host_tips = TipCodes(taxon_count, pattern_count, tips, tip_encoding, &engine->ambiguous);
     engine->host_weights = std::make_shared<std::vector<double>>(pattern_weights, pattern_weights + pattern_count);
   }
   if (const char* mode = std::getenv("SBNB_SUBSTITUTION_GRADIENT"))
@@ -1422,11 +1456,19 @@ int sbnb_device_count(void) {
 int sbnb_engine_create(const char* substitution, const char* site, const char* clock,
                        int32_t taxon_count, int64_t pattern_count, const uint8_t* tip_states,
                        const double* pattern_weights, int32_t device, sbnb_engine** out) {
+  return sbnb_engine_create_encoded(substitution, site, clock, taxon_count, pattern_count, tip_states,
+                                    SBNB_TIPS_STATES, pattern_weights, device, out);
+}
+
+int sbnb_engine_create_encoded(const char* substitution, const char* site, const char* clock,
+                               int32_t taxon_count, int64_t pattern_count, const uint8_t* tips,
+                               int32_t tip_encoding, const double* pattern_weights, int32_t device,
+                               sbnb_engine** out) {
   return Guard([&] {
     Require(out != nullptr, "NULL output handle.");
     *out = nullptr;
-    *out = CreateEngine(substitution, site, clock, taxon_count, pattern_count, tip_states, pattern_weights, device,
-                        nullptr)
+    *out = CreateEngine(substitution, site, clock, taxon_count, pattern_count, tips, tip_encoding, pattern_weights,
+                        device, nullptr)
                .release();
   });
 }
@@ -1435,6 +1477,14 @@ int sbnb_engine_create_multi(const char* substitution, const char* site, const c
                              int32_t taxon_count, int64_t pattern_count, const uint8_t* tip_states,
                              const double* pattern_weights, const int32_t* devices, int32_t device_count,
                              int32_t shard_axis, sbnb_engine** out) {
+  return sbnb_engine_create_multi_encoded(substitution, site, clock, taxon_count, pattern_count, tip_states,
+                                          SBNB_TIPS_STATES, pattern_weights, devices, device_count, shard_axis, out);
+}
+
+int sbnb_engine_create_multi_encoded(const char* substitution, const char* site, const char* clock,
+                                     int32_t taxon_count, int64_t pattern_count, const uint8_t* tips,
+                                     int32_t tip_encoding, const double* pattern_weights, const int32_t* devices,
+                                     int32_t device_count, int32_t shard_axis, sbnb_engine** out) {
   return Guard([&] {
     Require(out != nullptr, "NULL output handle.");
     *out = nullptr;
@@ -1445,8 +1495,8 @@ int sbnb_engine_create_multi(const char* substitution, const char* site, const c
     auto group = std::make_unique<sbnb_engine>();
     group->shard_axis = shard_axis;
     for (int g = 0; g < device_count; g++) {
-      auto child = CreateEngine(substitution, site, clock, taxon_count, pattern_count, tip_states, pattern_weights,
-                                devices[g], group->children.empty() ? nullptr : group->children[0]);
+      auto child = CreateEngine(substitution, site, clock, taxon_count, pattern_count, tips, tip_encoding,
+                                pattern_weights, devices[g], group->children.empty() ? nullptr : group->children[0]);
       if (shard_axis == SBNB_SHARD_PATTERNS && device_count > 1)
         UploadPatternRange(child.get(), pattern_count * g / device_count, pattern_count * (g + 1) / device_count);
       group->children.push_back(child.release());
@@ -1458,6 +1508,7 @@ int sbnb_engine_create_multi(const char* substitution, const char* site, const c
     group->pattern_count = first->pattern_count;
     group->categories = first->categories;
     group->padded_categories = first->padded_categories;
+    group->ambiguous = first->ambiguous;
     group->substitution_mode = first->substitution_mode;
     *out = group.release();
   });

@@ -1235,6 +1235,7 @@ struct sbnb_gp_engine {
       node_probabilities, inverted_prior;
   DeviceArray<double> matrix_cache;
   std::vector<uint8_t> host_tips;  // [taxon][pattern], for re-initialising the PLVs when the site model changes
+  bool tip_masks = false;          // host_tips are nucleotide masks (SBNB_TIPS_NUCLEOTIDE_MASKS), not states
   DeviceArray<int32_t> counts, program, status, tips;
   // programs seen before (the reference regenerates the same few schedules call after call)
   std::vector<std::unique_ptr<CompiledProgram>> compiled;
@@ -1467,7 +1468,9 @@ void SetCategories(sbnb_gp_engine* e, int categories, const double* rates, const
         const uint8_t symbol = e->host_tips[static_cast<size_t>(taxon) * P + k];
         for (int c = 0; c < categories; c++) {
           double* x = tips.data() + (static_cast<size_t>(taxon) * E + k * categories + c) * 4;
-          if (symbol == 4) {
+          if (e->tip_masks) {
+            for (int s = 0; s < 4; s++) x[s] = (symbol >> s) & 1 ? 1.0 : 0.0;  // 15: the all-ones gap
+          } else if (symbol == 4) {
             x[0] = x[1] = x[2] = x[3] = 1.0;
           } else if (symbol < 4) {
             x[symbol] = 1.0;
@@ -1724,11 +1727,28 @@ int sbnb_gp_create(int32_t taxon_count, int64_t pattern_count, const uint8_t* ti
                    double rescaling_threshold, const double* sbn_prior,
                    const double* unconditional_node_probabilities, int32_t node_count,
                    const double* inverted_sbn_prior, int32_t device, sbnb_gp_engine** out) {
+  return sbnb_gp_create_encoded(taxon_count, pattern_count, tip_states, SBNB_TIPS_STATES, pattern_weights,
+                                site_count, plv_count, gpcsp_count, rescaling_threshold, sbn_prior,
+                                unconditional_node_probabilities, node_count, inverted_sbn_prior, device, out);
+}
+
+int sbnb_gp_create_encoded(int32_t taxon_count, int64_t pattern_count, const uint8_t* tip_states, int32_t tip_encoding,
+                           const double* pattern_weights, int64_t site_count, int32_t plv_count,
+                           int32_t gpcsp_count, double rescaling_threshold, const double* sbn_prior,
+                           const double* unconditional_node_probabilities, int32_t node_count,
+                           const double* inverted_sbn_prior, int32_t device, sbnb_gp_engine** out) {
   return Guard([&] {
     Require(out != nullptr, "NULL output handle.");
     *out = nullptr;
     Require(taxon_count >= 1 && pattern_count >= 1, "Need at least 1 taxon and 1 site pattern.");
     Require(tip_states && pattern_weights, "NULL tip_states / pattern_weights.");
+    Require(tip_encoding == SBNB_TIPS_STATES || tip_encoding == SBNB_TIPS_NUCLEOTIDE_MASKS, "Unknown tip encoding.");
+    if (tip_encoding == SBNB_TIPS_NUCLEOTIDE_MASKS)
+      for (size_t i = 0; i < static_cast<size_t>(taxon_count) * pattern_count; i++)
+        if (tip_states[i] == 0 || tip_states[i] > 15)
+          Fail(SBNB_ERR_INVALID_ARGUMENT, "Invalid nucleotide mask " + std::to_string(tip_states[i]) + " at taxon " +
+                                              std::to_string(i / pattern_count) + ", pattern " +
+                                              std::to_string(i % pattern_count) + " (masks are 1..15).");
     Require(plv_count >= taxon_count, "plv_count must cover the taxa (6 PLVs per DAG node).");
     Require(gpcsp_count >= 0, "Negative GPCSP count.");
     Require(rescaling_threshold > 0.0 && rescaling_threshold < 1.0, "rescaling_threshold must be in (0, 1).");
@@ -1756,6 +1776,7 @@ int sbnb_gp_create(int32_t taxon_count, int64_t pattern_count, const uint8_t* ti
     const int64_t P = pattern_count;
     const size_t gpcsps = std::max(gpcsp_count, 1);
     e->host_tips.assign(tip_states, tip_states + static_cast<size_t>(taxon_count) * P);
+    e->tip_masks = tip_encoding == SBNB_TIPS_NUCLEOTIDE_MASKS;
     const double unit = 1.0;
     SetCategories(e.get(), 1, &unit, &unit);
     e->weights.Upload(pattern_weights, P, e->stream);

@@ -76,6 +76,24 @@ void BuildSymbolTable(uint8_t (&table)[256]) {
   for (const char* c = "-NX?BDHKMRSUVWY"; *c; c++) table[static_cast<unsigned char>(*c)] = 4;
 }
 
+// The IUPAC nucleotide codes as masks of the states they allow (bit 0 = A, 1 = C, 2 = G,
+// 3 = T), upper and lower case; U = T; N X ? - = 15 (missing).
+void BuildMaskTable(uint8_t (&table)[256]) {
+  std::memset(table, kUnknownSymbol, sizeof(table));
+  static const struct {
+    char symbol;
+    uint8_t mask;
+  } kCodes[] = {{'A', 1},  {'C', 2},  {'G', 4},  {'T', 8},  {'U', 8},  {'R', 5},  {'Y', 10}, {'S', 6},
+                {'W', 9},  {'K', 12}, {'M', 3},  {'B', 14}, {'D', 13}, {'H', 11}, {'V', 7},  {'N', 15},
+                {'X', 15}};
+  for (const auto& code : kCodes) {
+    table[static_cast<unsigned char>(code.symbol)] = code.mask;
+    table[static_cast<unsigned char>(code.symbol - 'A' + 'a')] = code.mask;
+  }
+  table[static_cast<unsigned char>('?')] = 15;
+  table[static_cast<unsigned char>('-')] = 15;
+}
+
 struct SymbolTable {
   uint8_t map[256];
 };
@@ -102,14 +120,19 @@ __device__ __forceinline__ uint32_t HashStep(uint32_t h, uint32_t word, uint32_t
 }
 
 // status[0] = 1 + an unknown character seen (0 = none); status[1] = collision flag.
+// MASKS: the table holds nucleotide masks 1..15, and an unknown character hashes as 0.
+template <bool MASKS>
 __global__ void __launch_bounds__(kHashThreads) HashKernel(
     const uint8_t* __restrict__ sequences, uint64_t* __restrict__ keys, int32_t taxon_count, int64_t site_count,
     int64_t pitch, uint64_t seed, uint64_t key_mask, const SymbolTable table, int32_t* __restrict__ status) {
   // character -> its symbol as a 4-bit field already in the place of taxon i of a group of 8
-  // (an unknown character: 0xf, the only value with bit 3 set)
+  // (an unknown character: 0xf, the only value with bit 3 set; with MASKS, 0, the only zero field)
   __shared__ uint32_t shifted[8][256];
-  for (int i = threadIdx.x; i < 8 * 256; i += blockDim.x)
-    shifted[i >> 8][i & 255] = static_cast<uint32_t>(table.map[i & 255] & 0xfu) << (4 * (i >> 8));
+  for (int i = threadIdx.x; i < 8 * 256; i += blockDim.x) {
+    const uint8_t symbol = table.map[i & 255];
+    const uint32_t field = MASKS ? (symbol == kUnknownSymbol ? 0u : symbol) : (symbol & 0xfu);
+    shifted[i >> 8][i & 255] = field << (4 * (i >> 8));
+  }
   __syncthreads();
   const int64_t group = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const int64_t site0 = group * kSitesPerThread;
@@ -124,7 +147,7 @@ __global__ void __launch_bounds__(kHashThreads) HashKernel(
     ha[k] = 0x811c9dc5u ^ seed_low;
     hb[k] = 0x9e3779b9u + seed_high;
   }
-  uint32_t seen = 0;  // OR of the packed words: bit 3 of a field = an unknown character
+  uint32_t seen = 0;  // bit 3 of a field = an unknown character (MASKS: of the zero-field test)
   const uint8_t* column = sequences + site0;
   for (int t0 = 0; t0 < taxon_count; t0 += 16) {
     // (a thread has one 4-byte load per taxon, so the loads of many taxa must be in flight
@@ -148,7 +171,9 @@ __global__ void __launch_bounds__(kHashThreads) HashKernel(
       }
 #pragma unroll
       for (int k = 0; k < kSitesPerThread; k++) {
-        seen |= packed[k];
+        // (MASKS: a field is zero exactly when it borrows in packed - 0x11111111 without having
+        //  had bit 3 set; the padding taxa of a group read as 'A' = 1)
+        seen |= MASKS ? (packed[k] - 0x11111111u) & ~packed[k] : packed[k];
         ha[k] = HashStep(ha[k], packed[k], 0xcc9e2d51u, 0x1b873593u, 15, 13, 5u, 0xe6546b64u);  // (MurmurHash3's own)
         hb[k] = HashStep(hb[k], packed[k], 0x85ebca6bu, 0xc2b2ae35u, 16, 11, 9u, 0x7f4a7c15u);
       }
@@ -396,7 +421,7 @@ __global__ void __launch_bounds__(256) TileKernel(const uint8_t* __restrict__ se
   if (VERIFY && difference != 0) status[1] = 1;
 }
 
-void Compress(int32_t n, int64_t S, const char* sequences, int32_t device, uint8_t* out_patterns,
+void Compress(int32_t n, int64_t S, const char* sequences, bool masks, int32_t device, uint8_t* out_patterns,
               double* out_weights, int64_t* out_pattern_count, double* out_device_ms) {
   Require(n > 0, "Site pattern compression needs at least one sequence.");
   Require(S >= 0 && S < (1ll << 30), "Site count out of range [0, 2^30).");  // 32-bit site ids, 2S-slot table
@@ -470,7 +495,11 @@ void Compress(int32_t n, int64_t S, const char* sequences, int32_t device, uint8
 
   stage("host -> device");
   SymbolTable table;
-  BuildSymbolTable(table.map);
+  if (masks) {
+    BuildMaskTable(table.map);
+  } else {
+    BuildSymbolTable(table.map);
+  }
   cudaEvent_t begin, end;
   SBNB_CUDA(cudaEventCreate(&begin));
   SBNB_CUDA(cudaEventCreate(&end));
@@ -499,7 +528,8 @@ void Compress(int32_t n, int64_t S, const char* sequences, int32_t device, uint8
     SBNB_CUDA(cudaMemset(d_table_count.get(), 0, static_cast<size_t>(table_size) * sizeof(uint32_t)));
     SBNB_CUDA(cudaEventRecord(begin));
     const int64_t groups = pitch / kSitesPerThread;
-    HashKernel<<<static_cast<int>((groups + kHashThreads - 1) / kHashThreads), kHashThreads>>>(
+    (masks ? HashKernel<true> : HashKernel<false>)<<<static_cast<int>((groups + kHashThreads - 1) / kHashThreads),
+                                                     kHashThreads>>>(
         d_sequences.get(), d_keys.get(), n, S, pitch, seed * 0x9e3779b97f4a7c15ull, key_mask, table, d_status.get());
     InsertKernel<<<site_blocks, 256>>>(d_keys.get(), d_table_keys.get(), d_table_first.get(),
                                        d_table_count.get(), d_slot_of.get(), S, table_size - 1);
@@ -567,7 +597,19 @@ extern "C" int sbnb_compress_site_patterns(int32_t taxon_count, int64_t site_cou
                                            int32_t device, uint8_t* out_patterns, double* out_weights,
                                            int64_t* out_pattern_count, double* out_device_ms) {
   return sbnb::Guard([&] {
-    sbnb::Compress(taxon_count, site_count, sequences, device, out_patterns, out_weights, out_pattern_count,
+    sbnb::Compress(taxon_count, site_count, sequences, false, device, out_patterns, out_weights, out_pattern_count,
                    out_device_ms);
+  });
+}
+
+extern "C" int sbnb_compress_site_patterns_encoded(int32_t taxon_count, int64_t site_count, const char* sequences,
+                                                   int32_t tip_encoding, int32_t device, uint8_t* out_patterns,
+                                                   double* out_weights, int64_t* out_pattern_count,
+                                                   double* out_device_ms) {
+  return sbnb::Guard([&] {
+    sbnb::Require(tip_encoding == SBNB_TIPS_STATES || tip_encoding == SBNB_TIPS_NUCLEOTIDE_MASKS,
+                  "Unknown tip encoding.");
+    sbnb::Compress(taxon_count, site_count, sequences, tip_encoding == SBNB_TIPS_NUCLEOTIDE_MASKS, device,
+                   out_patterns, out_weights, out_pattern_count, out_device_ms);
   });
 }

@@ -446,11 +446,25 @@ __host__ __device__ constexpr int OeStageBytes(int C, int K, bool subst = false)
 __host__ __device__ constexpr int OePreBatch(int K) { return K > 2 ? 2 : K; }
 // Read-back slots of one pre-order op: [warp][batch][child][j][half][lane] double2.
 __host__ __device__ constexpr int OeReadbackBytes(int K) { return 2 * K * 2 * kThreads * 16; }
-// model constants of the analytic substitution gradient: V, V^-1, and V^-1 e_s per tip state
-constexpr int kOeSubstSmemDoubles = 16 + 16 + 20;
-__host__ __device__ constexpr size_t OeSmemBytes(int C, int K, bool grad, bool subst = false) {
+// Tip codes.  An alignment given as nucleotide masks (bit 0 = A .. bit 3 = T) is held as
+// codes 0..3 (one state), 4 (all four: missing, also the padding) and 5..14 (the ten two-
+// and three-state masks, in ascending order of the mask).  Nibble c of kTipCodeMasks is
+// the mask of code c.  Codes 0..4 index the rows of a tip table directly; a walk
+// instantiated for ambiguous tips sums the state rows of codes 5..14.
+constexpr int kFirstAmbiguousCode = 5;
+constexpr int kTipCodes = 15;
+constexpr uint64_t kTipCodeMasks = 0xEDCBA97653F8421ull;
+__host__ __device__ constexpr unsigned TipCodeMask(int code) {
+  return static_cast<unsigned>(kTipCodeMasks >> (4 * code)) & 15u;
+}
+// model constants of the analytic substitution gradient: V, V^-1, and V^-1 L per tip code
+// (codes 0..4; all 15 codes in a walk over ambiguous tips)
+__host__ __device__ constexpr int OeTipZDoubles(bool ambig) { return 4 * (ambig ? kTipCodes : kFirstAmbiguousCode); }
+__host__ __device__ constexpr int OeSubstSmemDoubles(bool ambig) { return 16 + 16 + OeTipZDoubles(ambig); }
+__host__ __device__ constexpr size_t OeSmemBytes(int C, int K, bool grad, bool subst = false, bool ambig = false) {
   return static_cast<size_t>(OeStages(C, grad)) * OeStageBytes(C, K, subst) + 2 * OeStages(C, grad) * 8 +
-         (ModelSmemDoubles(C) + kOeSubstSmemDoubles) * 8 + 16 + 2 * kWarps * 8 + (grad ? OeReadbackBytes(K) : 0);
+         (ModelSmemDoubles(C) + OeSubstSmemDoubles(ambig)) * 8 + 16 + 2 * kWarps * 8 +
+         (grad ? OeReadbackBytes(K) : 0);
 }
 // Resident CTAs per SM the register allocation is held to.
 __host__ __device__ constexpr int OeMinBlocks(int K, bool grad, bool subst = false) {
@@ -540,7 +554,23 @@ __device__ __forceinline__ void NormalizeOe(double (&v)[K][4], int (&exps)[K]) {
   }
 }
 
-template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false>
+// y = the tip-table row(s) of the tip code of pattern j in `packed`: one row for codes 0..4,
+// the sum of the state rows of an ambiguous code (a tip's contribution M L_tip is linear in
+// L_tip, the indicator vector of its states).  Every lane loads the row of its code or of
+// the lowest state of its mask; lanes of ambiguous codes then add one or two more rows.
+__device__ __forceinline__ void LoadAmbiguousTipRow(const double* table, uint32_t packed, int j, double (&y)[4]) {
+  const int code = (packed >> (8 * j)) & 0xff;
+  const unsigned mask = code >= kFirstAmbiguousCode ? TipCodeMask(code) : 0u;
+  Load4(table + 4 * (mask != 0u ? __ffs(mask) - 1 : code), y);
+  for (unsigned rest = mask & (mask - 1); rest != 0u; rest &= rest - 1) {
+    double row[4];
+    Load4(table + 4 * (__ffs(rest) - 1), row);
+#pragma unroll
+    for (int i = 0; i < 4; i++) y[i] += row[i];
+  }
+}
+
+template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false, bool AMBIG = false>
 __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWalkOeKernel(const OeParams p) {
   static_assert(GRAD || !SUBST, "the substitution gradient rides on the pre-order pass");
   static_assert((C & (C - 1)) == 0 && C >= 1 && C <= 32, "lanes per pattern must be a power of two");
@@ -581,12 +611,13 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
   double* const rate_weight_smem = cat_weight_smem + ModelSmemCategories(C);
   double* const drate_weight_smem = rate_weight_smem + ModelSmemCategories(C);
   double* const freqs_smem = drate_weight_smem + ModelSmemCategories(C);
-  double* const evec_smem = freqs_smem + 4;  // V, V^-1 and V^-1 e_s (s = A C G T, gap): analytic substitution gradient
+  double* const evec_smem = freqs_smem + 4;  // V, V^-1 and V^-1 L per tip code: analytic substitution gradient
   double* const ivec_smem = evec_smem + 16;
   double* const tip_z_smem = ivec_smem + 16;
+  constexpr int kTipZ = OeTipZDoubles(AMBIG);
   // Sequence number of the next op whose operands have not been requested yet.
-  uint32_t* const ticket = reinterpret_cast<uint32_t*>(tip_z_smem + 20);
-  uint64_t* const readback_bars = reinterpret_cast<uint64_t*>(tip_z_smem + 22);
+  uint32_t* const ticket = reinterpret_cast<uint32_t*>(tip_z_smem + kTipZ);
+  uint64_t* const readback_bars = reinterpret_cast<uint64_t*>(tip_z_smem + kTipZ + 2);
   uint64_t* const readback_full = readback_bars + warp * 2;
   // Read-back slots, [warp][batch][child][j][half][lane] double2, filled per warp by
   // bulk copies that complete on the warp's own barriers.
@@ -641,12 +672,22 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
       rate_weight_smem[tid] = model.rates[tid];
       drate_weight_smem[tid] = model.drates[tid];
     }
-    if (SUBST && tid >= 32 && tid < 52) {
-      // V^-1 L for a tip: column s of V^-1 for a resolved state, the row sums for a gap
+    if (SUBST && tid >= 32 && tid < 32 + kTipZ) {
+      // V^-1 L for a tip: column s of V^-1 for a resolved state, the row sums for a gap,
+      // the sum of its states' columns for an ambiguous code
       const int state = (tid - 32) / 4, k = (tid - 32) % 4;
-      tip_z_smem[tid - 32] = state < 4 ? model.ivec[k * 4 + state]
-                                       : model.ivec[k * 4] + model.ivec[k * 4 + 1] + model.ivec[k * 4 + 2] +
-                                             model.ivec[k * 4 + 3];
+      if constexpr (AMBIG) {
+        if (state >= kFirstAmbiguousCode) {
+          double sum = 0.0;
+          for (int s = 0; s < 4; s++)
+            if (TipCodeMask(state) >> s & 1u) sum += model.ivec[k * 4 + s];
+          tip_z_smem[tid - 32] = sum;
+        }
+      }
+      if (!AMBIG || state < kFirstAmbiguousCode)
+        tip_z_smem[tid - 32] = state < 4 ? model.ivec[k * 4 + state]
+                                         : model.ivec[k * 4] + model.ivec[k * 4 + 1] + model.ivec[k * 4 + 2] +
+                                               model.ivec[k * 4 + 3];
     }
     if (GRAD) {
       // This warp owns its rows of edge-derivative sums for the whole item: clear them
@@ -784,6 +825,7 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
           return *at;
         };
         // doubles from the start of a category's tip table to the row of pattern j's state
+        // (AMBIG: LoadAmbiguousTipRow sums the state rows of an ambiguous code)
         auto tip_row = [](uint32_t packed, int j) -> int { return ((packed >> (8 * j)) & 0xff) * 4; };
         // The host orders the children of every op so that an internal child whose
         // partial is (post-order) or stays (pre-order) in cur is child a, and a child
@@ -823,7 +865,9 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
           if (a_leaf) {
             const uint32_t states_a = tip_states(tips_at);
 #pragma unroll
-            for (int j = 0; j < K; j++) Load4(operand + cat * kTipTableDoubles + tip_row(states_a, j), ya[j]);
+            for (int j = 0; j < K; j++)
+              if constexpr (AMBIG) LoadAmbiguousTipRow(operand + cat * kTipTableDoubles, states_a, j, ya[j]);
+              else Load4(operand + cat * kTipTableDoubles + tip_row(states_a, j), ya[j]);
             if (RESCALE) {
 #pragma unroll
               for (int j = 0; j < K; j++) cur_exp[j] = 0;
@@ -836,7 +880,9 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
           if (b_leaf) {
             const uint32_t states_b = tip_states(tips_at + kTipBytes);
 #pragma unroll
-            for (int j = 0; j < K; j++) Load4(part_b + cat * kTipTableDoubles + tip_row(states_b, j), yb[j]);
+            for (int j = 0; j < K; j++)
+              if constexpr (AMBIG) LoadAmbiguousTipRow(part_b + cat * kTipTableDoubles, states_b, j, yb[j]);
+              else Load4(part_b + cat * kTipTableDoubles + tip_row(states_b, j), yb[j]);
           } else {
             const int s2 = (record.y >> 16) & 0xff;
             double x[K][4];
@@ -938,7 +984,8 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
             if (a_leaf) {
 #pragma unroll
               for (int j = 0; j < KP; j++)
-                Load4(table_a + cat * kTipTableDoubles + tip_row(states_a, j0 + j), ya[j]);
+                if constexpr (AMBIG) LoadAmbiguousTipRow(table_a + cat * kTipTableDoubles, states_a, j0 + j, ya[j]);
+                else Load4(table_a + cat * kTipTableDoubles + tip_row(states_a, j0 + j), ya[j]);
             } else {
               const double2* const slot_a = slot + ((swapped && !b_leaf) ? KP * 64 : 0);
 #pragma unroll
@@ -950,7 +997,8 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
             if (b_leaf) {
 #pragma unroll
               for (int j = 0; j < KP; j++)
-                Load4(table_b + cat * kTipTableDoubles + tip_row(states_b, j0 + j), yb[j]);
+                if constexpr (AMBIG) LoadAmbiguousTipRow(table_b + cat * kTipTableDoubles, states_b, j0 + j, yb[j]);
+                else Load4(table_b + cat * kTipTableDoubles + tip_row(states_b, j0 + j), yb[j]);
             } else {
               const double2* const slot_b = slot + (swapped ? 0 : KP * 64);
 #pragma unroll
@@ -1016,7 +1064,8 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
 #pragma unroll
               for (int j = 0; j < KP; j++) {
                 double d[4];
-                Load4(table_a + (C + cat) * kTipTableDoubles + tip_row(states_a, j0 + j), d);
+                if constexpr (AMBIG) LoadAmbiguousTipRow(table_a + (C + cat) * kTipTableDoubles, states_a, j0 + j, d);
+                else Load4(table_a + (C + cat) * kTipTableDoubles + tip_row(states_a, j0 + j), d);
                 g_a = fma(scale[j], Dot4(top[j], d), g_a);
               }
               if (SUBST) {
@@ -1055,7 +1104,8 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
 #pragma unroll
               for (int j = 0; j < KP; j++) {
                 double d[4];
-                Load4(table_b + (C + cat) * kTipTableDoubles + tip_row(states_b, j0 + j), d);
+                if constexpr (AMBIG) LoadAmbiguousTipRow(table_b + (C + cat) * kTipTableDoubles, states_b, j0 + j, d);
+                else Load4(table_b + (C + cat) * kTipTableDoubles + tip_row(states_b, j0 + j), d);
                 g_b = fma(scale[j], Dot4(yb[j], d), g_b);
               }
               if (SUBST) {

@@ -137,30 +137,36 @@ class StagedBatch:
 class Engine:
     """B200 likelihood engine for one alignment and one phylo-model specification."""
 
-    def __init__(self, specification, patterns, weights, device=0, devices=None, shard_axis="trees"):
+    def __init__(self, specification, patterns, weights, device=0, devices=None, shard_axis="trees",
+                 tip_encoding="states"):
         """device: one CUDA ordinal; or devices=[...]: a device group inside the library
         (sbnb_engine_create_multi: one host thread + stream per GPU), sharded by
-        "trees" or by "patterns" (SURVEY.md 8e)."""
+        "trees" or by "patterns" (SURVEY.md 8e).  tip_encoding: "states" (0..3 = ACGT,
+        anything >= 4 a gap) or "masks" (nucleotide masks, bit 0 = A .. bit 3 = T: an
+        ambiguous character such as R = 5 enters as the partial vector of its states)."""
         lib = _capi.load()
+        encoding = _capi.tip_encoding(tip_encoding)
         patterns = np.ascontiguousarray(patterns, dtype=np.uint8)
         weights = np.ascontiguousarray(weights, dtype=np.float64)
         if patterns.ndim != 2 or weights.shape != (patterns.shape[1],):
             raise RuntimeError("patterns must be [taxon][pattern] and weights [pattern].")
         self.specification = specification
+        self.tip_encoding = tip_encoding
         self.taxon_count, self.pattern_count = patterns.shape
         handle = ctypes.c_void_p()
         common = (specification.substitution.encode(), specification.site.encode(),
                   specification.clock.encode(), self.taxon_count, self.pattern_count,
                   patterns.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)), _capi.as_double_ptr(weights))
+        common = common[:6] + (encoding,) + common[6:]
         if devices is None:
-            _capi.check(lib.sbnb_engine_create(*common, device, ctypes.byref(handle)))
+            _capi.check(lib.sbnb_engine_create_encoded(*common, device, ctypes.byref(handle)))
         else:
             if shard_axis not in ("trees", "patterns"):
                 raise RuntimeError("shard_axis must be 'trees' or 'patterns'.")
             ordinals = np.ascontiguousarray(devices, dtype=np.int32)
             axis = _capi.SHARD_TREES if shard_axis == "trees" else _capi.SHARD_PATTERNS
-            _capi.check(lib.sbnb_engine_create_multi(*common, _capi.as_int32_ptr(ordinals), len(ordinals), axis,
-                                                     ctypes.byref(handle)))
+            _capi.check(lib.sbnb_engine_create_multi_encoded(*common, _capi.as_int32_ptr(ordinals), len(ordinals),
+                                                             axis, ctypes.byref(handle)))
             device = int(ordinals[0])
         self._handle = handle
         self.device = device

@@ -93,8 +93,11 @@ class GPEngine:
 
     def __init__(self, tip_states, pattern_weights, site_count, plv_count, gpcsp_count,
                  rescaling_threshold=default_rescaling_threshold, sbn_prior=None,
-                 unconditional_node_probabilities=None, inverted_sbn_prior=None, device=0):
+                 unconditional_node_probabilities=None, inverted_sbn_prior=None, device=0, tip_encoding="states"):
+        """tip_encoding: "states" (0..3 = ACGT, 4 = gap) or "masks" (nucleotide masks 1..15:
+        leaf PLV entry s = bit s of the tip's mask)."""
         self._lib = _capi.load()
+        encoding = _capi.tip_encoding(tip_encoding)
         tip_states = np.ascontiguousarray(tip_states, dtype=np.uint8)
         if tip_states.ndim != 2:
             raise ValueError("tip_states must be [taxon][pattern]")
@@ -118,9 +121,9 @@ class GPEngine:
         prior = optional(sbn_prior, self.gpcsp_count, "sbn_prior")
         inverted = optional(inverted_sbn_prior, self.gpcsp_count, "inverted_sbn_prior")
         handle = ctypes.c_void_p()
-        _capi.check(self._lib.sbnb_gp_create(
+        _capi.check(self._lib.sbnb_gp_create_encoded(
             self.taxon_count, self.pattern_count, tip_states.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)),
-            _capi.as_double_ptr(weights), int(site_count), self.plv_count, self.gpcsp_count,
+            encoding, _capi.as_double_ptr(weights), int(site_count), self.plv_count, self.gpcsp_count,
             float(rescaling_threshold), _capi.as_double_ptr(prior), _capi.as_double_ptr(nodes), self.node_count,
             _capi.as_double_ptr(inverted), int(device), ctypes.byref(handle)))
         self._handle = handle

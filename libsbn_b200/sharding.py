@@ -104,9 +104,9 @@ class TreeShardedEngine:
     """Engine whose batch calls evaluate this rank's slice of the trees and
     all-gather the per-tree results, so every rank returns the whole batch."""
 
-    def __init__(self, specification, patterns, weights, device=0):
+    def __init__(self, specification, patterns, weights, device=0, tip_encoding="states"):
         self.rank, self.world, self.backend = _world()
-        self.engine = Engine(specification, patterns, weights, device)
+        self.engine = Engine(specification, patterns, weights, device, tip_encoding=tip_encoding)
 
     def local_slice(self, trees, params):
         begin, end = shard_range(self.rank, self.world, trees.tree_count)
@@ -234,13 +234,13 @@ class PatternShardedEngine:
     """Engine restricted to this rank's range of site patterns; batch calls walk
     ALL trees over the local patterns and sum-all-reduce the raw results."""
 
-    def __init__(self, specification, patterns, weights, device=0, presharded=False):
+    def __init__(self, specification, patterns, weights, device=0, presharded=False, tip_encoding="states"):
         """presharded: `patterns` / `weights` are already this rank's columns only (an
         alignment too large to build on every rank); otherwise every rank passes the
-        whole alignment and keeps its range of it."""
+        whole alignment and keeps its range of it.  tip_encoding as for Engine."""
         self.rank, self.world, self.backend = _world()
         self.specification = specification
-        self.engine = Engine(specification, patterns, weights, device)
+        self.engine = Engine(specification, patterns, weights, device, tip_encoding=tip_encoding)
         if presharded:
             self.begin, self.end = 0, self.engine.pattern_count
         else:

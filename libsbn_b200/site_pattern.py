@@ -5,6 +5,9 @@ device through sbnb_compress_site_patterns (include/sbn_b200_patterns.h).
     pattern = SitePattern(sequences)          # list of equal-length strings, leaf-id order,
                                               # or a C-contiguous uint8 array [taxon][site] of characters
     engine = Engine(spec, pattern.patterns, pattern.weights)
+
+    pattern = SitePattern(sequences, ambiguity=True)   # IUPAC nucleotide masks
+    engine = Engine(spec, pattern.patterns, pattern.weights, tip_encoding="masks")
 """
 import ctypes
 
@@ -14,10 +17,11 @@ from . import _capi
 
 
 class SitePattern:
-    """patterns: uint8 [taxon][pattern] (0..3 = ACGT, 4 = gap), weights: float64
-    [pattern]; patterns are in order of first appearance in the alignment."""
+    """patterns: uint8 [taxon][pattern] (0..3 = ACGT, 4 = gap; with ambiguity=True the
+    IUPAC nucleotide masks 1..15), weights: float64 [pattern]; patterns are in order of
+    first appearance in the alignment."""
 
-    def __init__(self, sequences, device=0):
+    def __init__(self, sequences, device=0, ambiguity=False):
         if isinstance(sequences, np.ndarray) and sequences.ndim == 2 and sequences.dtype == np.uint8:
             # the characters as they lie in memory: no host copy
             keep = np.ascontiguousarray(sequences)
@@ -37,9 +41,11 @@ class SitePattern:
         patterns = np.empty(max(len(rows) * length, 1), dtype=np.uint8)
         weights = np.empty(max(length, 1), dtype=np.float64)
         count, device_ms = ctypes.c_int64(), ctypes.c_double()
-        _capi.check(_capi.load().sbnb_compress_site_patterns(
-            len(rows), length, flat, device, patterns.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)),
+        encoding = _capi.TIPS_NUCLEOTIDE_MASKS if ambiguity else _capi.TIPS_STATES
+        _capi.check(_capi.load().sbnb_compress_site_patterns_encoded(
+            len(rows), length, flat, encoding, device, patterns.ctypes.data_as(ctypes.POINTER(ctypes.c_uint8)),
             _capi.as_double_ptr(weights), ctypes.byref(count), ctypes.byref(device_ms)))
+        self.ambiguity = ambiguity
         self.pattern_count = count.value
         # (no second copy of an alignment that did not shrink)
         self.patterns = patterns[:len(rows) * count.value].reshape(len(rows), count.value)

@@ -122,6 +122,36 @@ def random_alignment(taxon_count, pattern_count, seed, gap_fraction=0.01):
     return states, np.ones(pattern_count)
 
 
+def random_masked_alignment(taxon_count, pattern_count, seed, ambiguous_fraction=0.05, gap_fraction=0.01):
+    """Nucleotide masks (bit 0 = A .. bit 3 = T): iid uniform single states, a fraction
+    of missing characters (15) and a fraction of ambiguous ones drawn uniformly from the
+    ten two- and three-state masks; every column its own pattern with weight 1."""
+    rng = np.random.default_rng(seed)
+    masks = (1 << rng.integers(0, 4, size=(taxon_count, pattern_count))).astype(np.uint8)
+    draw = rng.random((taxon_count, pattern_count))
+    masks[draw < gap_fraction] = 15
+    ambiguous = (draw >= gap_fraction) & (draw < gap_fraction + ambiguous_fraction)
+    choices = np.array([3, 5, 6, 7, 9, 10, 11, 12, 13, 14], dtype=np.uint8)
+    masks[ambiguous] = choices[rng.integers(0, len(choices), size=int(ambiguous.sum()))]
+    return masks, np.ones(pattern_count)
+
+
+def states_to_masks(states):
+    """States (0..3, >= 4 gap) -> the equivalent nucleotide masks (1, 2, 4, 8, 15)."""
+    states = np.asarray(states)
+    return np.where(states < 4, np.left_shift(1, np.minimum(states, 3)), 15).astype(np.uint8)
+
+
+def masks_to_states(masks):
+    """Masks -> states, every ambiguous mask turned into a gap (what the state table keeps)."""
+    masks = np.asarray(masks)
+    single = {1: 0, 2: 1, 4: 2, 8: 3}
+    out = np.full(masks.shape, 4, dtype=np.uint8)
+    for mask, state in single.items():
+        out[masks == mask] = state
+    return out
+
+
 def newick(parent_ids, branch_lengths, taxon_names=None):
     """Newick string of one tree (children in id order, lengths by node id)."""
     node_count = len(parent_ids) + 1
