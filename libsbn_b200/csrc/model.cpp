@@ -115,7 +115,7 @@ int ModelSpec::SubstitutionGradientSize() const {
     case SubstitutionKind::kGTR:
       return 8;
     case SubstitutionKind::kHKY:
-      return 4;  // kappa (log space) + 3 frequency coordinates
+      return 4;  // kappa (linear) + 3 frequency coordinates
     default:
       return 0;
   }

@@ -219,10 +219,17 @@ __global__ void TransitionMatrixOeKernel(const OeMatrixParams p) {
       double row[4];
 #pragma unroll
       for (int l = 0; l < 4; l++) {
-        // e^{l_l tau} tau (e^x - 1) / x,  x = (l_k - l_l) tau
+        // int_0^tau e^{l_k s} e^{l_l (tau - s)} ds, x = (l_k - l_l) tau, from the larger
+        // exponent: e^{l_k tau} tau (1 - e^-x) / x if x > 0, else e^{l_l tau} tau (e^x - 1) / x.
+        // (e^x - 1 overflows for x > 709 and e^{l_l tau} underflows on long branches.)
         const double x = (model.eval[k] - model.eval[l]) * t;
-        const double ratio = fabs(x) < 1e-8 ? 1.0 + 0.5 * x : expm1(x) / x;
-        row[l] = ex[l] * t * ratio;
+        if (x > 0.0) {
+          const double ratio = x < 1e-8 ? 1.0 - 0.5 * x : -expm1(-x) / x;
+          row[l] = ex[k] * t * ratio;
+        } else {
+          const double ratio = x > -1e-8 ? 1.0 + 0.5 * x : expm1(x) / x;
+          row[l] = ex[l] * t * ratio;
+        }
       }
       out[2 * k] = make_double2(row[0], row[1]);
       out[2 * k + 1] = make_double2(row[2], row[3]);
