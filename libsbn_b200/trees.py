@@ -113,6 +113,63 @@ def random_tree_batch(taxon_count, tree_count, seed, mean_branch_length=0.1, roo
     return parent_ids, lengths
 
 
+def random_time_trees(taxon_count, tree_count, seed, epochs=4, relaxed=False, ladder=False, topology_count=None):
+    """Seeded dated (time) trees: a dict of everything TreeBatch takes.
+
+    Tips are sampled at `epochs` dates, so internal nodes both share their bound with an
+    internal child and sit above a child of an older epoch; internal bounds are the
+    largest bound of their children.  A non-root node d internal nodes above its deepest
+    tip has ratio (d + u) / (d + 1), u uniform in [-0.5, 0.5], clipped to [1e-3, 0.999]:
+    the ratios on a path then multiply to about (d + 1) / (depth + 1), so even a 1000-taxon
+    ladder keeps every branch far from 0 (a product of independent ratios would shrink
+    geometrically, and fp64 transition matrices of branches near 1e-9 are only good to
+    ~1e-16 / length, which decides the likelihood of alignments with a change on every
+    branch).  Then
+    heights follow top-down as h = b + r (h_parent - b) (the float64 expression any
+    reference must repeat to see the same heights); height_ratios[n - 2] is the root
+    height, branch_lengths[e] = h_parent - h_e with the root's entry 0.  Strict clock:
+    one rate c != 1 on every edge (rate_count 1); relaxed: lognormal rates per edge
+    (rate_count 2n - 2).  topology_count: reuse that many topologies cyclically, each
+    tree with its own dates, ratios and rates; ladder: caterpillar topologies."""
+    rng = np.random.default_rng(seed)
+    n, N = taxon_count, 2 * taxon_count - 1
+    shapes = topology_count or tree_count
+    topologies = [ladder_topology(n, unrooted=False) if ladder else random_rooted_topology(n, rng)
+                  for _ in range(shapes)]
+    out = {name: np.zeros((tree_count, width)) for name, width in (
+        ("branch_lengths", N), ("rates", N - 1), ("node_heights", N), ("node_bounds", N), ("height_ratios", n - 1))}
+    out["parent_ids"] = np.stack([topologies[t % shapes] for t in range(tree_count)])
+    out["rate_count"] = N - 1 if relaxed else 1
+    for t in range(tree_count):
+        parent = out["parent_ids"][t]
+        children = [[] for _ in range(N)]
+        for child, p in enumerate(parent):
+            children[p].append(child)
+        dates = np.concatenate([[0.0], np.cumsum(rng.uniform(0.02, 0.1, size=epochs - 1))])
+        for _ in range(100):  # until both sides of the epoch test occur (where the shape allows)
+            bounds = np.zeros(N)
+            bounds[:n] = dates[rng.integers(0, epochs, size=n)]
+            for node in range(n, N):
+                bounds[node] = max(bounds[c] for c in children[node])
+            pairs = [(bounds[node] == bounds[c]) for node in range(n, N - 1) for c in children[node] if c >= n]
+            if epochs < 2 or (any(pairs) and not all(pairs)):
+                break
+        above = np.zeros(N)
+        for node in range(n, N):
+            above[node] = 1 + max(above[c] for c in children[node])
+        ratios = np.clip((above[n:] + rng.uniform(-0.5, 0.5, size=n - 1)) / (above[n:] + 1), 1e-3, 0.999)
+        ratios[n - 2] = bounds[N - 1] + rng.uniform(0.2, 0.6)
+        heights = bounds.copy()
+        heights[N - 1] = ratios[n - 2]
+        for node in range(N - 2, n - 1, -1):
+            heights[node] = bounds[node] + ratios[node - n] * (heights[parent[node]] - bounds[node])
+        out["branch_lengths"][t, :N - 1] = heights[parent] - heights[:N - 1]
+        clock = rng.choice([rng.uniform(0.4, 0.9), rng.uniform(1.1, 1.6)])
+        out["rates"][t] = clock * (rng.lognormal(0.0, 0.4, size=N - 1) if relaxed else 1.0)
+        out["node_heights"][t], out["node_bounds"][t], out["height_ratios"][t] = heights, bounds, ratios
+    return out
+
+
 def random_alignment(taxon_count, pattern_count, seed, gap_fraction=0.01):
     """iid uniform {A,C,G,T} with a fraction of gap states; every column is kept
     as its own pattern with weight 1 (BASELINE config 4/5 shape)."""

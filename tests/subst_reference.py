@@ -100,43 +100,35 @@ def tip_vectors(tips, masks):
     return np.where(tips[..., None] >= 4, 1.0, (tips[..., None] == np.arange(4)).astype(np.float64))
 
 
-def log_likelihood_and_gradient(substitution, site, tips, weights, parent_ids, lengths, params, masks=False):
-    """(logL, d logL / d coordinates in the engine's order) of one tree.
+def prune(qs, freqs, category_rates, category_weights, tips, weights, parent_ids, lengths, masks=False):
+    """Per-evaluation logL of J complex evaluations of one tree, batched on a leading axis.
 
-    tips: [taxon][pattern]; parent_ids: [nodes - 1]; lengths: [nodes] (the root's entry is
-    unused); params: the substitution and site blocks of an engine parameter row."""
-    params = np.asarray(params, dtype=np.float64)
-    base, model = coordinates(substitution, params)
-    shape = params[10 if substitution == "GTR" else 5] if site != "constant" else None
-    rates, category_weights = site_rates(site, shape)
-    J = len(base)
-    # one complex evaluation per coordinate, batched on a leading axis
-    qs, freqs = [], []
-    for j in range(J):
-        y = np.array(base, dtype=np.complex128)
-        y[j] += 1j * STEP
-        exchangeabilities, pi = model(list(y))
-        qs.append(rate_matrix(exchangeabilities, pi))
-        freqs.append(pi)
-    qs, freqs = np.array(qs), np.array(freqs, dtype=np.complex128)  # [J][4][4], [J][4]
+    qs: [J][4][4] rate matrices; freqs: [J][4]; category_rates: [C] or [J][C], or
+    [J][edge][C] for rates that differ per edge; category_weights: [C]; lengths: [nodes]
+    or [J][nodes] (the root's entry is unused)."""
+    J = len(qs)
     parent_ids = np.asarray(parent_ids)
-    lengths = np.asarray(lengths, dtype=np.float64)
     node_count = len(parent_ids) + 1
-    taxa = np.asarray(tips).shape[0]
-    tau = lengths[:node_count - 1, None] * rates[None, :]  # [edge][C]
-    transition = scipy.linalg.expm(qs[:, None, None] * tau[None, :, :, None, None])  # [J][edge][C][4][4]
+    taxa, pattern_count = np.asarray(tips).shape
+    lengths = np.broadcast_to(np.asarray(lengths)[..., :node_count - 1], (J, node_count - 1))
+    category_rates = np.asarray(category_rates)
+    if category_rates.ndim < 3:
+        category_rates = np.broadcast_to(category_rates, (J, len(category_weights)))[:, None, :]
+    tau = lengths[:, :, None] * category_rates  # [J][edge][C]
+    transition = scipy.linalg.expm(qs[:, None, None] * tau[:, :, :, None, None])  # [J][edge][C][4][4]
+    C = tau.shape[2]
     leaves = tip_vectors(tips, masks)
     children = [[] for _ in range(node_count)]
     for child, parent in enumerate(parent_ids):
         children[parent].append(child)
-    partial, log_scale = {}, np.zeros((J, np.asarray(tips).shape[1]))
+    partial, log_scale = {}, np.zeros((J, pattern_count))
     for node in range(taxa, node_count):  # every child id is smaller than its parent's
         product = None
         for child in children[node]:
             below = partial.pop(child) if child >= taxa else leaves[child][None, None]
             # (P L)[j, c, p, i] = sum_s P[j, c, i, s] L[j, c, p, s]
-            evolved = np.einsum("jcis,jcps->jcpi", transition[:, child], np.broadcast_to(
-                below, (J, len(rates)) + below.shape[2:]))
+            evolved = np.matmul(np.broadcast_to(below, (J, C) + below.shape[2:]),
+                                transition[:, child].swapaxes(-1, -2))
             product = evolved if product is None else product * evolved
         # a real factor per pattern: the complex step is untouched and 1000 taxa do not underflow
         scale = np.max(product.real, axis=(1, 3))
@@ -144,7 +136,35 @@ def log_likelihood_and_gradient(substitution, site, tips, weights, parent_ids, l
         partial[node] = product / scale[:, None, :, None]
         log_scale += np.log(scale)
     root = partial.pop(node_count - 1)
-    site_likelihood = np.einsum("c,jcps,js->jp", category_weights, root, freqs)
+    site_likelihood = np.einsum("c,jcps,js->jp", category_weights, root, np.asarray(freqs, dtype=np.complex128))
     per_site = np.log(site_likelihood) + log_scale
-    total = per_site @ np.asarray(weights, dtype=np.float64)
+    return per_site @ np.asarray(weights, dtype=np.float64)
+
+
+def model_at(substitution, params, base, step):
+    """(Q [J][4][4], pi [J][4]): one evaluation per coordinate, that coordinate stepped by i * step."""
+    _, model = coordinates(substitution, params)
+    qs, freqs = [], []
+    for j in range(len(base)):
+        y = np.array(base, dtype=np.complex128)
+        y[j] += 1j * step
+        exchangeabilities, pi = model(list(y))
+        qs.append(rate_matrix(exchangeabilities, pi))
+        freqs.append(pi)
+    return np.array(qs), np.array(freqs, dtype=np.complex128)
+
+
+def log_likelihood_and_gradient(substitution, site, tips, weights, parent_ids, lengths, params, masks=False):
+    """(logL, d logL / d coordinates in the engine's order) of one tree.
+
+    tips: [taxon][pattern]; parent_ids: [nodes - 1]; lengths: [nodes] (the root's entry is
+    unused); params: the substitution and site blocks of an engine parameter row."""
+    params = np.asarray(params, dtype=np.float64)
+    base, _ = coordinates(substitution, params)
+    shape = params[10 if substitution == "GTR" else 5] if site != "constant" else None
+    rates, category_weights = site_rates(site, shape)
+    # one complex evaluation per coordinate, batched on a leading axis
+    qs, freqs = model_at(substitution, params, base, STEP)
+    total = prune(qs, freqs, rates, category_weights, tips, weights, parent_ids,
+                  np.asarray(lengths, dtype=np.float64), masks)
     return float(total[0].real), total.imag / STEP

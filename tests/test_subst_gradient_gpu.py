@@ -20,6 +20,7 @@ from conftest import load_fixture
 import libsbn_b200 as sbn
 from libsbn_b200 import _capi, sharding, trees
 import subst_reference as ref
+import time_tree_reference as tt
 
 pytestmark = pytest.mark.gpu
 
@@ -52,19 +53,48 @@ def synthetic(taxa=21, patterns=509, seed=3, masks=False):
     return tips, weights
 
 
-def check(got, substitution, site, tips, weights, parent_ids, lengths, params, masks=False, references=None):
-    """Every tree of `got` against the reference; returns the references for reuse."""
+def check(got, substitution, site, tips, weights, parent_ids, lengths, params, masks=False, references=None,
+          branches=True):
+    """Every tree of `got` against the reference; returns the references for reuse.  With
+    `branches`, also the branch-length and site-model blocks against
+    time_tree_reference.unrooted_gradient (the complex step on every edge and the shape)."""
     references = references or [
         ref.log_likelihood_and_gradient(substitution, site, tips, weights, parent_ids[t], lengths[t], params[t],
-                                        masks=masks) for t in range(len(got))]
-    for t, (g, (logl, want)) in enumerate(zip(got, references)):
+                                        masks=masks) +
+        (tt.unrooted_gradient(substitution, site, tips, weights, parent_ids[t], lengths[t], params[t], masks)[1:]
+         if branches else (None, None)) for t in range(len(got))]
+    for t, (g, (logl, want, branch, shape)) in enumerate(zip(got, references)):
         a = g.gradient["substitution_model"]
         assert a.shape == want.shape
         assert np.all(np.isfinite(a)), f"tree {t}: {a}"
         assert abs(g.log_likelihood - logl) <= LOGL_RTOL * abs(logl), f"tree {t}"
         error = np.max(np.abs(a - want)) / np.max(np.abs(want))
         assert error <= SUBST_RTOL, f"tree {t}: relative error {error:.3e}\n{a}\n{want}"
+        if branch is not None:
+            check_branches(g.gradient["branch_lengths"], branch, parent_ids[t], t)
+        if shape is not None:
+            assert abs(g.gradient["site_model"][0] - shape) <= SUBST_RTOL * abs(shape), f"tree {t}: site model"
     return references
+
+
+def check_branches(a, want, parent_ids, t):
+    """The engine's [2n-1] branch-length block against d logL / d (each edge of the tree as
+    given).  A trifurcating tree keeps its edge ids, the two edges detrifurcation adds get 0;
+    a bifurcating tree's root slide puts the root edge's derivative on the first child of the
+    root and 0 on the second, so the two are compared as a sum (each side of the root edge
+    has that derivative: the pulley principle)."""
+    edges = len(parent_ids)
+    root_children = np.flatnonzero(np.asarray(parent_ids) == edges)
+    scale = np.max(np.abs(want))
+    if len(root_children) == 3:
+        assert np.all(a[edges:] == 0.0)
+        error = np.max(np.abs(a[:edges] - want)) / scale
+    else:
+        first, second = root_children
+        rest = np.setdiff1d(np.arange(edges), root_children)
+        error = max(np.max(np.abs(a[rest] - want[rest])), abs(a[first] + a[second] - want[first]),
+                    abs(a[first] + a[second] - want[second])) / scale
+    assert error <= SUBST_RTOL, f"tree {t}: branch lengths, relative error {error:.3e}"
 
 
 def run_both_modes(engine, batch, params, rooted=False):
@@ -119,7 +149,7 @@ def test_time_trees(substitution, site):
     references = None
     for got in run_both_modes(engine, batch, params, rooted=True):
         references = check(got, substitution, site, fx["patterns"], fx["weights"], fx["parent_ids"], effective,
-                           params, references=references)
+                           params, references=references, branches=False)
 
 
 @pytest.mark.parametrize("shape,substitution,site", [
@@ -136,7 +166,7 @@ def test_thousand_taxa_rescaled(shape, substitution, site):
     params = np.array([random_row(substitution, site, rng)])
     engine = sbn.Engine(sbn.PhyloModelSpecification(substitution, site, "none"), tips, weights)
     got = engine.gradients(sbn.TreeBatch(parent_ids, lengths), params, True)
-    check(got, substitution, site, tips, weights, parent_ids, lengths, params)
+    check(got, substitution, site, tips, weights, parent_ids, lengths, params, branches=False)
 
 
 @pytest.mark.parametrize("site", ["weibull+4", "weibull+32"])

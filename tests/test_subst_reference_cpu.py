@@ -25,8 +25,9 @@ def mp_stick_breaking(y):
     return x + [stick]
 
 
-def mp_log_likelihood(substitution, site, tips, weights, parent_ids, lengths, shape, y):
-    """logL at the coordinates y, every step at DIGITS digits."""
+def mp_log_likelihood(substitution, site, tips, weights, parent_ids, lengths, shape, y, category_rates=None):
+    """logL at the coordinates y, every step at DIGITS digits (lengths may be mpf; Weibull
+    category rates from the shape unless category_rates gives them)."""
     if substitution == "GTR":
         exchangeabilities, freqs = mp_stick_breaking(y[:5]), mp_stick_breaking(y[5:8])
     else:
@@ -41,7 +42,9 @@ def mp_log_likelihood(substitution, site, tips, weights, parent_ids, lengths, sh
     for i in range(4):
         q[i, i] = -sum(q[i, j] for j in range(4) if j != i)
     q /= -sum(freqs[i] * q[i, i] for i in range(4))
-    if site == "constant":
+    if category_rates is not None:
+        rates = list(category_rates)
+    elif site == "constant":
         rates = [mpmath.mpf(1)]
     else:
         count = int(site.split("+")[1])
@@ -55,7 +58,7 @@ def mp_log_likelihood(substitution, site, tips, weights, parent_ids, lengths, sh
     for child, parent in enumerate(parent_ids):
         children[parent].append(child)
     total = mpmath.mpf(0)
-    matrices = [[mpmath.expm(q * (mpmath.mpf(float(lengths[e])) * r)) for r in rates] for e in range(node_count - 1)]
+    matrices = [[mpmath.expm(q * (mpmath.mpf(lengths[e]) * r)) for r in rates] for e in range(node_count - 1)]
     for p in range(len(weights)):
         site_likelihood = mpmath.mpf(0)
         for c in range(len(rates)):
