@@ -163,6 +163,24 @@ def random_tree_operations(n, rng, rescaling, order="libsbn"):
     return np.array(post, dtype=np.int32), np.array(pre, dtype=np.int32)
 
 
+def depth_first_operations(post, n):
+    """The same ops, children before parents in depth-first order (libsbn's traversal order: the
+    destination of an op is a child of the next one, which the device kernel keeps in registers)."""
+    by_dest = {int(op[0]): op for op in post}
+    order, stack = [], [(int(post[-1][0]), False)]
+    while stack:  # (no recursion: a 1000-taxon ladder is 999 ops deep)
+        v, expanded = stack.pop()
+        if v < n:
+            continue
+        if expanded:
+            order.append(by_dest[v])
+        else:
+            stack.append((v, True))
+            stack.append((int(by_dest[v][5]), False))
+            stack.append((int(by_dest[v][3]), False))
+    return np.array(order, dtype=np.int32)
+
+
 def gtr_eigensystem():
     rates = np.array([0.05, 0.1, 0.15, 0.20, 0.25, 0.25])
     freqs = np.array([0.1, 0.2, 0.3, 0.4])

@@ -21,7 +21,8 @@ import pytest
 from conftest import ROOT
 import test_integration_gpu as integration
 
-from libsbn_b200.beagle import Beagle, LIB_PATH as SHIM, gtr_eigensystem, random_tree_operations
+from libsbn_b200.beagle import (Beagle, LIB_PATH as SHIM, depth_first_operations, gtr_eigensystem,
+                                random_tree_operations)
 
 ORACLE = os.path.join(ROOT, "oracle", "_build", "libbeagle_oracle.so")
 
@@ -91,23 +92,6 @@ def test_reference_doctest_suite_passes_over_the_device_beagle_library():
     assert b"beagleUpdatePrePartials" in binary  # the reference's FatBeagle is what runs
 
 
-def _depth_first(post, n):
-    """The same ops, children before parents in depth-first order (libsbn's traversal order: the
-    destination of an op is a child of the next one, which the device kernel keeps in registers)."""
-    by_dest = {int(op[0]): op for op in post}
-    order = []
-
-    def visit(v):
-        if v < n:
-            return
-        visit(int(by_dest[v][3]))
-        visit(int(by_dest[v][5]))
-        order.append(by_dest[v])
-
-    visit(int(post[-1][0]))
-    return np.array(order, dtype=np.int32)
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("categories,variant", [(4, "depth_first"), (4, "cumulative_is_written"), (2, "depth_first"),
                                                 (8, "depth_first"), (1, "both_children_forwarded")])
@@ -122,7 +106,7 @@ def test_partial_update_op_lists_the_pipelined_kernel_special_cases(categories, 
     states[rng.random(states.shape) < 0.05] = 4
     weights = rng.integers(1, 4, size=P).astype(np.float64)
     post, _ = random_tree_operations(n, rng, True, "node_id")
-    post = _depth_first(post, n)
+    post = depth_first_operations(post, n)
     assert len(post) == n - 1 > 32
     if variant == "cumulative_is_written":
         post[5][1] = 0
