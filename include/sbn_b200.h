@@ -59,7 +59,12 @@ int sbnb_device_count(void);
  * (fat_beagle.cpp:13-29): model specification strings as in
  * PhyloModelSpecification (phylo_model.hpp:13-17):
  *   substitution: "JC69" | "GTR" | "HKY"  (HKY is an addition; see DESIGN.md)
- *   site:         "constant" | "weibull+K" | "weibull" (K=4)
+ *   site:         "constant" | "weibull+K" | "weibull" (K=4) | "gamma+K" | "gamma", each
+ *                 optionally followed by "+I": a proportion p of invariable sites,
+ *                 lik = (1 - p) L(rates / (1 - p)) + p I with I the summed frequencies of
+ *                 the states every tip of the pattern allows (DESIGN.md, K2); p is the
+ *                 last entry of the "entire site" block ("proportion invariant"), and any p
+ *                 outside [0, 1) fails with SBNB_ERR_MODEL
  *   clock:        "none" | "strict"
  * tip_states is SitePattern::GetPatterns() flattened [taxon][pattern]
  * (site_pattern.hpp:46-50): 0..3 = A,C,G,T, anything >= 4 = gap/unknown.
@@ -137,8 +142,8 @@ int32_t sbnb_engine_device_count(const sbnb_engine* engine);
 
 /* Engine::GetPhyloModelBlockSpecification (engine.hpp:31): total parameter
  * count K of one row, and (start, length) of a named block such as
- * "GTR rates", "frequencies", "kappa", "Weibull shape", "Gamma shape", "clock rate", "entire
- * substitution", "entire site", "entire clock".  Unknown key -> error. */
+ * "GTR rates", "frequencies", "kappa", "Weibull shape", "Gamma shape", "proportion invariant",
+ * "clock rate", "entire substitution", "entire site", "entire clock".  Unknown key -> error. */
 int32_t sbnb_engine_param_count(const sbnb_engine* engine);
 int sbnb_engine_param_block(const sbnb_engine* engine, const char* key, int32_t* start,
                             int32_t* length);
@@ -165,7 +170,8 @@ typedef struct {
   double* log_likelihood;     /* [T]                                            */
   double* branch_lengths;     /* [T][2n-1]   "branch_lengths"  (unrooted only)  */
   double* substitution_model; /* [T][8]      "substitution_model" (GTR; HKY: 4) */
-  double* site_model;         /* [T][1]      "site_model"      (categories > 1) */
+  double* site_model;         /* [T][site entries] "site_model": the shape (categories > 1), then
+                                 d/d proportion invariant (+I); 1 entry for every model without +I */
   double* ratios_root_height; /* [T][n-1]    "ratios_root_height" (rooted only) */
   double* clock_model;        /* [T][rate_count] "clock_model"    (rooted only) */
 } sbnb_gradient_out;
@@ -232,6 +238,11 @@ int sbnb_batch_fetch(sbnb_engine* engine, sbnb_batch* batch, double* log_likelih
  * SBNB_STAGE_SUBSTITUTION_ANALYTIC: [T][20] = W (16, row-major) then R (4).  Sums over site
  * patterns: ranks that each hold a pattern range add them like the other raw results. */
 int sbnb_batch_fetch_substitution_sums(sbnb_engine* engine, sbnb_batch* batch, double* sums);
+/* The sums of the invariant class of the last gradient run of a +I model: [T][5] = D, then
+ * E_A..E_T (DESIGN.md, K2; E only in batches staged with SBNB_STAGE_SUBSTITUTION_ANALYTIC, else 0).
+ * Sums over site patterns: ranks that each hold a pattern range add them like the other raw
+ * results (on the device they follow the substitution sums in the result array). */
+int sbnb_batch_fetch_invariant_sums(sbnb_engine* engine, sbnb_batch* batch, double* sums);
 /* Device addresses of the raw result arrays sbnb_batch_fetch copies out
  * (fp64: [evaluation_count], [T][2n-1], [T][2n-1]), valid until the batch is
  * destroyed.  For site-pattern sharding: the ranks sum-all-reduce these in
@@ -292,6 +303,17 @@ int sbnb_finish_gradients_analytic(const char* substitution, const char* site, c
                                    const double* params, const double* log_likelihoods,
                                    const double* branch_gradients, const double* rate_gradients,
                                    const double* substitution_sums, const sbnb_gradient_out* out);
+/* The host tail for a +I site model, which the two entries above refuse (they have no
+ * d/d proportion invariant): everything as sbnb_finish_gradients_analytic, with the [T][5]
+ * sums of sbnb_batch_fetch_invariant_sums; substitution_sums may be NULL (no
+ * "substitution_model" block is then written).  The site-model row is [shape | proportion
+ * invariant]: d logL / dp = D + sum over edges of tau g / (1 - p). */
+int sbnb_finish_gradients_invariant(const char* substitution, const char* site, const char* clock,
+                                    int32_t taxon_count, const sbnb_tree_batch* trees, int32_t rooted,
+                                    const double* params, const double* log_likelihoods,
+                                    const double* branch_gradients, const double* rate_gradients,
+                                    const double* substitution_sums, const double* invariant_sums,
+                                    const sbnb_gradient_out* out);
 /* Adds the log-determinant Jacobian of the height-ratio transform
  * (fat_beagle.cpp:82-94) to already reduced rooted log-likelihoods, in place. */
 int sbnb_finish_log_likelihoods_rooted(int32_t taxon_count, const sbnb_tree_batch* trees,
@@ -310,7 +332,8 @@ int sbnb_debug_tree_program(const int32_t* parent_ids, int32_t node_count, int32
 
 /* The model tables built from one parameter row: eigenvectors[16],
  * inverse_eigenvectors[16], eigenvalues[4], frequencies[4], q[16] (row-major),
- * then category rates / weights / rate derivatives (category_count each). */
+ * then category rates / weights / rate derivatives (category_count each; with +I the rates
+ * and their derivatives divided by 1 - proportion invariant). */
 int sbnb_debug_model_tables(const char* substitution, const char* site, const char* clock,
                             const double* param_row, double* eigenvectors,
                             double* inverse_eigenvectors, double* eigenvalues, double* frequencies,

@@ -94,6 +94,11 @@ SIGNATURES = {
                                                   _P(TreeBatchStruct), _c.c_int32, _P(_c.c_double), _P(_c.c_double),
                                                   _P(_c.c_double), _P(_c.c_double), _P(_c.c_double),
                                                   _P(GradientOutStruct)]),
+    "sbnb_batch_fetch_invariant_sums": (_c.c_int, [_c.c_void_p, _c.c_void_p, _P(_c.c_double)]),
+    "sbnb_finish_gradients_invariant": (_c.c_int, [_c.c_char_p, _c.c_char_p, _c.c_char_p, _c.c_int32,
+                                                   _P(TreeBatchStruct), _c.c_int32, _P(_c.c_double), _P(_c.c_double),
+                                                   _P(_c.c_double), _P(_c.c_double), _P(_c.c_double), _P(_c.c_double),
+                                                   _P(GradientOutStruct)]),
     "sbnb_finish_gradients": (_c.c_int, [_c.c_char_p, _c.c_char_p, _c.c_char_p, _c.c_int32, _P(TreeBatchStruct),
                                          _c.c_int32, _c.c_int32, _P(_c.c_double), _P(_c.c_double),
                                          _P(_c.c_double), _P(GradientOutStruct)]),
@@ -160,6 +165,7 @@ STAGE_ROOTED = 1
 STAGE_SUBSTITUTION_FD = 2
 STAGE_SUBSTITUTION_ANALYTIC = 4
 SUBSTITUTION_SUMS = 20
+INVARIANT_SUMS = 5  # +I: D, then E_A..E_T (sbnb_batch_fetch_invariant_sums)
 SHARD_TREES = 0
 TIPS_STATES = 0
 TIPS_NUCLEOTIDE_MASKS = 1

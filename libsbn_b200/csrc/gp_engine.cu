@@ -1944,6 +1944,7 @@ int sbnb_gp_set_site_model(sbnb_gp_engine* e, const char* site, const double* pa
   return Guard([&] {
     Require(e != nullptr && site != nullptr, "NULL argument.");
     const ModelSpec spec = ModelSpec::Parse("JC69", site, "none");
+    Require(!spec.invariant, "The GP engine has no invariable-site (+I) model.");
     Require(param_count == spec.param_count,
             std::string("The ") + site + " site model takes " + std::to_string(spec.param_count) + " parameters.");
     Require(params != nullptr || param_count == 0, "NULL parameters.");

@@ -35,6 +35,29 @@ void CheckCategoryCount(const ModelSpec& spec, const std::string& site) {
              "BEAGLE-compatible device library behind the unmodified FatBeagle, takes any number)");
 }
 
+// "weibull" / "gamma" (4 categories) or "weibull+K" / "gamma+K" with K all digits.
+int CategoryCount(const std::string& base, const std::string& name, const std::string& site) {
+  if (base == name) return 4;
+  const std::string digits = base.substr(std::min(base.size(), name.size() + 1));
+  if (base.compare(0, name.size() + 1, name + "+") != 0 || digits.empty() || digits.size() > 9 ||
+      digits.find_first_not_of("0123456789") != std::string::npos)
+    Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);
+  return std::stoi(digits);
+}
+
+// The "entire site" block: the shape (if any), then "proportion invariant" for +I.
+void AppendSiteBlock(ModelSpec* spec, const char* shape_key) {
+  std::vector<std::pair<std::string, int>> sub_blocks;
+  if (shape_key) sub_blocks.push_back({shape_key, 1});
+  const int start = spec->param_count;
+  AppendBlock(spec, "entire site", sub_blocks);
+  if (spec->invariant) {
+    spec->blocks["proportion invariant"] = {spec->param_count, 1};
+    spec->param_count += 1;
+    spec->blocks["entire site"] = {start, spec->param_count - start};
+  }
+}
+
 }  // namespace
 
 ModelSpec ModelSpec::Parse(const std::string& substitution, const std::string& site,
@@ -53,40 +76,27 @@ ModelSpec ModelSpec::Parse(const std::string& substitution, const std::string& s
     // substitution_model.cpp:14
     Fail(SBNB_ERR_INVALID_ARGUMENT, "Substitution model not known: " + substitution);
   }
-  if (site == "constant") {
+  // "<site>+I": the suffix is split off before the category count is read, so that
+  // "weibull+4+I" is Weibull with 4 categories and a proportion invariant.
+  const bool invariant = site.size() >= 2 && site.compare(site.size() - 2, 2, "+I") == 0;
+  const std::string base = invariant ? site.substr(0, site.size() - 2) : site;
+  spec.invariant = invariant;
+  if (base == "constant") {
     spec.site = SiteKind::kConstant;
     spec.category_count = 1;
-    AppendBlock(&spec, "entire site", {});
+    AppendSiteBlock(&spec, nullptr);
   } else if (site.rfind("weibull", 0) == 0) {
     // site_model.cpp:15-22: "weibull" (4 categories) or "weibull+K".
     spec.site = SiteKind::kWeibull;
-    spec.category_count = 4;
-    const auto plus = site.find('+');
-    if (plus != std::string::npos) {
-      try {
-        spec.category_count = std::stoi(site.substr(plus + 1));
-      } catch (const std::exception&) {
-        Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);
-      }
-    }
+    spec.category_count = CategoryCount(base, "weibull", site);
     CheckCategoryCount(spec, site);
-    AppendBlock(&spec, "entire site", {{"Weibull shape", 1}});
+    AppendSiteBlock(&spec, "Weibull shape");
   } else if (site.rfind("gamma", 0) == 0) {
     // Not in the reference (its "Gamma-4" is weibull+4): "gamma" (4 categories) or "gamma+K".
     spec.site = SiteKind::kGamma;
-    spec.category_count = 4;
-    const auto plus = site.find('+');
-    if (plus != std::string::npos) {
-      try {
-        spec.category_count = std::stoi(site.substr(plus + 1));
-      } catch (const std::exception&) {
-        Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);
-      }
-    } else if (site != "gamma") {
-      Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);
-    }
+    spec.category_count = CategoryCount(base, "gamma", site);
     CheckCategoryCount(spec, site);
-    AppendBlock(&spec, "entire site", {{"Gamma shape", 1}});
+    AppendSiteBlock(&spec, "Gamma shape");
   } else {
     Fail(SBNB_ERR_INVALID_ARGUMENT, "Site model not known: " + site);
   }
@@ -108,6 +118,11 @@ std::pair<int, int> ModelSpec::Block(const std::string& key) const {
   if (it == blocks.end())
     Fail(SBNB_ERR_INVALID_ARGUMENT, "Can't find block key: " + key);
   return it->second;
+}
+
+int ModelSpec::SiteGradientSize() const {
+  const int entries = (site == SiteKind::kConstant ? 0 : 1) + (invariant ? 1 : 0);
+  return entries > 0 ? entries : 1;
 }
 
 int ModelSpec::SubstitutionGradientSize() const {
@@ -332,7 +347,9 @@ double InverseRegularizedGammaP(double a, double p) {
   return x;
 }
 
-void BuildSite(const ModelSpec& spec, const double* params, ModelTables* out) {
+namespace {
+
+void BuildRateCategories(const ModelSpec& spec, const double* params, ModelTables* out) {
   const int count = spec.category_count;
   for (int c = 0; c < kMaxCategories; c++) {
     out->rates[c] = 1.0;
@@ -384,6 +401,23 @@ void BuildSite(const ModelSpec& spec, const double* params, ModelTables* out) {
                      (mean_rate * mean_rate);
     out->rates[i] /= mean_rate;
     out->weights[i] = 1.0 / count;  // site_model.hpp:57-59
+  }
+}
+
+}  // namespace
+
+void BuildSite(const ModelSpec& spec, const double* params, ModelTables* out) {
+  BuildRateCategories(spec, params, out);
+  out->pinv = 0.0;
+  if (!spec.invariant) return;
+  const double p = params[spec.Block("proportion invariant").first - spec.Block("entire site").first];
+  if (!(p >= 0.0 && p < 1.0)) Fail(SBNB_ERR_MODEL, "Proportion invariant must lie in [0, 1).");
+  out->pinv = p;
+  if (p == 0.0) return;  // (bitwise the tables of the site model without +I)
+  // The variable sites carry the whole substitution rate: mean rate over all sites 1.
+  for (int c = 0; c < spec.category_count; c++) {
+    out->rates[c] /= 1.0 - p;
+    out->drates[c] /= 1.0 - p;
   }
 }
 

@@ -22,6 +22,8 @@ struct ModelSpec {
   SiteKind site = SiteKind::kConstant;
   ClockKind clock = ClockKind::kNone;
   int category_count = 1;
+  // "<site>+I": a proportion of invariable sites, the last entry of the "entire site" block
+  bool invariant = false;
   int param_count = 0;
   // key -> (start, length); same keys the python block map shows.
   std::map<std::string, std::pair<int, int>> blocks;
@@ -32,6 +34,9 @@ struct ModelSpec {
   // Number of stick-breaking coordinates the finite-difference substitution
   // gradient runs over (GTR: 5 rates + 3 frequencies; fat_beagle.cpp:440-465).
   int SubstitutionGradientSize() const;
+  // Entries of one tree's "site_model" gradient row: the shape (Weibull, Gamma), then the
+  // proportion invariant (+I); 1 for a constant site model without +I (always 0).
+  int SiteGradientSize() const;
 };
 
 // The fused tree walk gives every rate category of a site pattern its own lane, so a
@@ -50,6 +55,8 @@ struct ModelTables {
   double rates[kMaxCategories];     // category rates r_c           (first category_count used)
   double weights[kMaxCategories];   // category proportions p_c
   double drates[kMaxCategories];    // d r_c / d shape (Weibull, Gamma; 0 for a constant site model)
+  double pinv;                      // proportion of invariable sites (+I; 0 otherwise).  rates and
+                                    // drates are then divided by 1 - pinv: the mean rate stays 1
 };
 
 // substitution_model.cpp:17-80 (GTR), substitution_model.hpp:59-74 (JC69).

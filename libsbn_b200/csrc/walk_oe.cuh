@@ -104,6 +104,8 @@ struct OeParams {
   double* grad_partial;    // [vtree][chunk][warp][2n-1]               (gradient mode)
   double* rgrad_partial;   // same, with d rate_c / d shape as the scalers (C > 1)
   double* subst_partial;   // [vtree][chunk][warp][kOeSubstSums]        (analytic substitution gradient)
+  const uint8_t* invariant_masks;  // [tip_pitch] the states every tip allows, per pattern (+I; 0 = padding)
+  double* inv_partial;     // [vtree][chunk][warp][kOeInvariantSums]    (+I gradient runs)
 };
 
 // ---------------------------------------------------------------------------
@@ -257,20 +259,37 @@ __global__ void TransitionMatrixOeKernel(const OeMatrixParams p) {
 }
 
 constexpr int kOeSubstSums = 20;  // W (16) and R (4) of the analytic substitution gradient
+// +I: D = sum of w (I - L) / lik and E_s = sum over the patterns whose tips all allow s of w / lik
+constexpr int kOeInvariantSums = 5;
 
-// One launch for all three result arrays: out = [logl (logl_count) | grad (rows x width) |
-// rgrad (rows x width)], each entry the fixed-order sum of its `parts` per-(chunk, warp)
+// One launch for all result arrays: out = [logl (logl_count) | grad (rows x width) |
+// rgrad (rows x width) | substitution sums (rows x kOeSubstSums) | +I sums (rows x
+// kOeInvariantSums)], each entry the fixed-order sum of its `parts` per-(chunk, warp)
 // partial rows (bitwise deterministic run to run).
 __global__ void ReduceAllKernel(const double* __restrict__ logl_partial, const double* __restrict__ grad_partial,
                                 const double* __restrict__ rgrad_partial, const double* __restrict__ subst_partial,
                                 double* __restrict__ out, int32_t logl_begin, int32_t logl_count,
-                                int32_t logl_total, int32_t grad_rows, int32_t width, int32_t parts) {
+                                int32_t logl_total, int32_t grad_rows, int32_t width, int32_t parts,
+                                const double* __restrict__ inv_partial = nullptr) {
   int64_t idx = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
   const int64_t grad_count = static_cast<int64_t>(grad_rows) * width;
+  const int64_t subst_count = static_cast<int64_t>(grad_rows) * kOeSubstSums;
+  if (inv_partial != nullptr && idx >= logl_count + 2 * grad_count + subst_count) {
+    // the +I sums: [tree][kOeInvariantSums] after the substitution sums
+    idx -= logl_count + 2 * grad_count + subst_count;
+    if (idx >= static_cast<int64_t>(grad_rows) * kOeInvariantSums) return;
+    const int64_t row = idx / kOeInvariantSums;
+    const int e = static_cast<int>(idx % kOeInvariantSums);
+    const double* src = inv_partial + row * parts * kOeInvariantSums + e;
+    double sum = 0.0;
+    for (int part = 0; part < parts; part++) sum += src[static_cast<int64_t>(part) * kOeInvariantSums];
+    out[logl_total + 2 * grad_count + subst_count + idx] = sum;
+    return;
+  }
   if (subst_partial != nullptr && idx >= logl_count + 2 * grad_count) {
     // the substitution-gradient sums: [tree][kOeSubstSums] after the three arrays
     idx -= logl_count + 2 * grad_count;
-    if (idx >= static_cast<int64_t>(grad_rows) * kOeSubstSums) return;
+    if (idx >= subst_count) return;
     const int64_t row = idx / kOeSubstSums;
     const int e = static_cast<int>(idx % kOeSubstSums);
     const double* src = subst_partial + row * parts * kOeSubstSums + e;
@@ -288,7 +307,7 @@ __global__ void ReduceAllKernel(const double* __restrict__ logl_partial, const d
     return;
   }
   int64_t k = idx - logl_count;
-  if (k >= 2 * grad_count) return;
+  if (k >= 2 * grad_count) return;  // (a substitution-sum index of a run without them)
   const double* partial = grad_partial;
   double* dst = out + logl_total;
   if (k >= grad_count) {
@@ -321,7 +340,13 @@ struct RootedFinishParams {
   const double* grad;        // [tree][2n-1] edge derivatives
   const double* rgrad;       // [tree][2n-1] or NULL (one category)
   double* scratch;           // [tree][5][n-1]
-  double* out;               // [tree][(n-1) + rate_count + 1]: ratios / root height, clock, site model
+  double* out;               // [tree][(n-1) + rate_count + site_width]: ratios / root height, clock, site model
+  // +I: the reduced [tree][kOeInvariantSums] sums and each tree's pinv, else NULL; the site-model
+  // row is then [shape (if any) | proportion invariant]
+  const double* inv_sums;
+  const ModelTables* models;
+  const int32_t* vtree_model;
+  int32_t site_width;
 };
 
 __global__ void RootedFinishKernel(const RootedFinishParams p) {
@@ -341,7 +366,8 @@ __global__ void RootedFinishKernel(const RootedFinishParams p) {
   double* log_time = chain + (n - 1);
   double* jacobian = log_time + (n - 1);
   double* multiplier = jacobian + (n - 1);
-  double* out = p.out + static_cast<size_t>(t) * (n - 1 + p.rate_count + 1);
+  const int site_width = p.inv_sums != nullptr ? p.site_width : 1;
+  double* out = p.out + static_cast<size_t>(t) * (n - 1 + p.rate_count + site_width);
 
   auto node_partial = [&](int node) { return (heights[node] - bounds[node]) / ratios[node - n]; };
   auto epoch_addition = [&](int node, int child, const double* ratio_gradient) {
@@ -406,6 +432,15 @@ __global__ void RootedFinishKernel(const RootedFinishParams p) {
     for (int node = 0; node < N - 1; node++) site += rg[node] * scaled[node];
   }
   out[n - 1 + p.rate_count] = site;
+  if (p.inv_sums != nullptr) {
+    // d logL / d pinv = D + sum over edges of tau g / (1 - pinv): the rates are divided by 1 - pinv
+    const double* scaled = p.scaled_lengths + static_cast<size_t>(t) * N;
+    double normalisation = 0.0;
+    for (int node = 0; node < N - 1; node++) normalisation += g[node] * scaled[node];
+    const double pinv = p.models[p.vtree_model[t]].pinv;
+    out[n - 1 + p.rate_count + site_width - 1] =
+        p.inv_sums[static_cast<size_t>(t) * kOeInvariantSums] + normalisation / (1.0 - pinv);
+  }
 }
 
 // Device groups sharded by site pattern (engine.cu): the raw per-tree sums of the other
@@ -463,6 +498,18 @@ constexpr int kTipCodes = 15;
 constexpr uint64_t kTipCodeMasks = 0xEDCBA97653F8421ull;
 __host__ __device__ constexpr unsigned TipCodeMask(int code) {
   return static_cast<unsigned>(kTipCodeMasks >> (4 * code)) & 15u;
+}
+// +I: per site pattern the set of states every tip allows (the AND of the tips' masks; a gap
+// allows all four), one byte per pattern beside the weights.  One thread per pattern of the
+// padded range, reading the [taxon][pattern] codes coalesced; the padding gets the empty set.
+__global__ void InvariantMaskKernel(const uint8_t* __restrict__ tips, int64_t tip_pitch, int32_t taxon_count,
+                                    int64_t pattern_count, uint8_t* __restrict__ masks) {
+  const int64_t k = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (k >= tip_pitch) return;
+  unsigned mask = 15u;
+  for (int taxon = 0; taxon < taxon_count && mask != 0u; taxon++)
+    mask &= TipCodeMask(tips[static_cast<int64_t>(taxon) * tip_pitch + k]);
+  masks[k] = static_cast<uint8_t>(k < pattern_count ? mask : 0u);
 }
 // model constants of the analytic substitution gradient: V, V^-1, and V^-1 L per tip code
 // (codes 0..4; all 15 codes in a walk over ambiguous tips)
@@ -577,7 +624,34 @@ __device__ __forceinline__ void LoadAmbiguousTipRow(const double* table, uint32_
   }
 }
 
-template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false, bool AMBIG = false>
+// A proportion pinv of invariable sites (+I): lik = (1 - pinv) L + pinv I, with L = site 2^exp
+// the mixture over the rate categories and I the summed frequencies of the states every tip
+// of the pattern allows.  Everything is a function of rho = I / L formed in the scaled
+// domain, so that neither 0 x inf nor inf / inf arises when L is far below the fp64 range:
+//   x = pinv rho / (1 - pinv),  f = (1 - pinv) L / lik = 1 / (1 + x),
+//   L / lik = f / (1 - pinv),   I / lik = rho f / (1 - pinv) = 1 / (pinv (1 + 1 / x)).
+// At pinv = 0 the log-likelihood and f are bitwise those of the model without +I.
+struct InvariantSiteTerms {
+  double log_lik, f, inv_over_lik, var_over_lik;
+};
+__device__ __forceinline__ InvariantSiteTerms InvariantSite(double log_l, double site, int exp, double pinv,
+                                                            double invariant) {
+  const double rho = invariant == 0.0 ? 0.0 : ldexp(invariant / site, -exp);
+  const double x = pinv == 0.0 ? 0.0 : pinv * rho / (1.0 - pinv);
+  InvariantSiteTerms t;
+  t.f = 1.0 / (1.0 + x);
+  t.var_over_lik = t.f / (1.0 - pinv);
+  if (x <= 1.0) {
+    t.log_lik = log_l + log1p(-pinv) + log1p(x);
+    t.inv_over_lik = rho * t.var_over_lik;
+  } else {  // (rho may be inf: the variable part is then below the fp64 range)
+    t.log_lik = log(pinv * invariant) + log1p(1.0 / x);
+    t.inv_over_lik = 1.0 / (pinv * (1.0 + 1.0 / x));
+  }
+  return t;
+}
+
+template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false, bool AMBIG = false, bool INVAR = false>
 __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWalkOeKernel(const OeParams p) {
   static_assert(GRAD || !SUBST, "the substitution gradient rides on the pre-order pass");
   static_assert((C & (C - 1)) == 0 && C >= 1 && C <= 32, "lanes per pattern must be a power of two");
@@ -703,6 +777,7 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
         grad_row[e] = 0.0;
         if (C > 1) rgrad_row[e] = 0.0;
       }
+      if (INVAR && lane < kOeInvariantSums) p.inv_partial[out_row * kOeInvariantSums + lane] = 0.0;
     }
     const int tile_begin = chunk * p.tiles_per_chunk;
     const int tile_end = min(tile_begin + p.tiles_per_chunk, p.tiles_total);
@@ -912,6 +987,16 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
             // beagleCalculateRootLogLikelihoods: log sum_c p_c sum_i pi_i L[c,k,i] (+ scale)
             double freqs[4];
             Load4(freqs_smem, freqs);
+            uint32_t masks = 0;  // +I: the states all tips allow, one byte per pattern
+            double pinv = 0.0;
+            // +I gradient runs: this tile's D and E_s (E only for the analytic substitution gradient)
+            double dinv = 0.0, einv[SUBST ? 4 : 1] = {};
+            if constexpr (INVAR) {
+              const uint8_t* const at = p.invariant_masks + pat0 + pidx * K;
+              masks = K == 4 ? *reinterpret_cast<const uint32_t*>(at)
+                             : (K == 2 ? *reinterpret_cast<const uint16_t*>(at) : *at);
+              pinv = model.pinv;
+            }
 #pragma unroll
             for (int j = 0; j < K; j++) {
               double site = cat_weight * Dot4(freqs, cur[j]);
@@ -919,8 +1004,47 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
               for (int s = kPerWarp; s < 32; s <<= 1) site += __shfl_xor_sync(0xffffffffu, site, s);
               double log_site = log(site);
               if (RESCALE) log_site = fma(static_cast<double>(cur_exp[j]), 0.6931471805599453094, log_site);
+              InvariantSiteTerms inv{};
+              double invariant = 0.0;
+              if constexpr (INVAR) {
+                const unsigned mask = (masks >> (8 * j)) & 15u;
+#pragma unroll
+                for (int s = 0; s < 4; s++)
+                  if (mask >> s & 1u) invariant += freqs[s];
+                inv = InvariantSite(log_site, site, RESCALE ? cur_exp[j] : 0, pinv, invariant);
+                log_site = inv.log_lik;
+              }
               // one lane per pattern carries the term
               logl_acc = fma(w[j], (w[j] != 0.0 && cat == 0) ? log_site : 0.0, logl_acc);
+              if constexpr (INVAR && GRAD) {
+                if (w[j] != 0.0 && cat == 0) {
+                  dinv += w[j] * (inv.inv_over_lik - inv.var_over_lik);
+                  if constexpr (SUBST) {
+                    const unsigned mask = (masks >> (8 * j)) & 15u;
+                    const double share = invariant > 0.0 ? w[j] * inv.inv_over_lik / invariant : 0.0;
+#pragma unroll
+                    for (int s = 0; s < 4; s++)
+                      if (mask >> s & 1u) einv[SUBST ? s : 0] += share;
+                  }
+                }
+                // every derivative of the variable part is weighted by f = (1 - pinv) L / lik:
+                // the pre-order pass below forms all of them from w
+                w[j] *= inv.f;
+              }
+            }
+            if constexpr (INVAR && GRAD) {
+              // added to the warp's row at once (single writer, in tile order), so that no
+              // accumulator stays live through the pre-order pass
+              double* const sums = p.inv_partial + out_row * kOeInvariantSums;
+              const double d_total = WarpSum(dinv);
+              if (lane == 0) sums[0] += d_total;
+              if constexpr (SUBST) {
+#pragma unroll
+                for (int s = 0; s < 4; s++) {
+                  const double e_total = WarpSum(einv[s]);
+                  if (lane == 0) sums[1 + s] += e_total;
+                }
+              }
             }
             if (GRAD) {
               // The pre-order pass starts at the root with T = p_c pi (its operand block

@@ -119,6 +119,13 @@ class StagedBatch:
                                                                     _capi.as_double_ptr(sums)))
         return sums
 
+    def fetch_invariant_sums(self):
+        """[T][5] sums of the invariant class (D, E_A..E_T) of the last gradient run of a +I model."""
+        sums = np.empty((self.tree_count, _capi.INVARIANT_SUMS))
+        _capi.check(_capi.load().sbnb_batch_fetch_invariant_sums(self._engine._handle, self._handle,
+                                                                 _capi.as_double_ptr(sums)))
+        return sums
+
     def algorithmic_bytes(self, mode):
         return _capi.load().sbnb_batch_algorithmic_bytes(self._handle, mode)
 
@@ -174,6 +181,9 @@ class Engine:
         self.substitution_gradient_mode = "fd" if os.environ.get("SBNB_SUBSTITUTION_GRADIENT") == "fd" else "analytic"
         self.param_count = lib.sbnb_engine_param_count(handle)
         self.category_count = lib.sbnb_engine_category_count(handle)
+        self.invariant = specification.site.endswith("+I")
+        # entries of a tree's "site_model" gradient: [shape | proportion invariant]
+        self.site_gradient_size = max(1, self.param_block("entire site")[1])
 
     def set_substitution_gradient(self, mode):
         """'analytic' (default): exact d logL / d (substitution parameters) inside the
@@ -206,8 +216,8 @@ class Engine:
     def param_block_map(self, params):
         """Views into a trees x params matrix by block name (get_phylo_model_param_block_map)."""
         out = {}
-        for key in ("GTR rates", "frequencies", "kappa", "Weibull shape", "Gamma shape", "clock rate",
-                    "entire substitution", "entire site", "entire clock", "entire"):
+        for key in ("GTR rates", "frequencies", "kappa", "Weibull shape", "Gamma shape", "proportion invariant",
+                    "clock rate", "entire substitution", "entire site", "entire clock", "entire"):
             try:
                 start, length = self.param_block(key)
             except _capi.SbnbError:
@@ -262,8 +272,8 @@ class Engine:
             buffers["branch_lengths"] = np.zeros((T, 2 * n - 1))
         if fd_size:
             buffers["substitution_model"] = np.zeros((T, fd_size))
-        if self.category_count > 1:
-            buffers["site_model"] = np.zeros((T, 1))
+        if self.category_count > 1 or self.invariant:
+            buffers["site_model"] = np.zeros((T, self.site_gradient_size))
         out = _capi.GradientOutStruct()
         for key, value in buffers.items():
             setattr(out, key, _capi.as_double_ptr(value))

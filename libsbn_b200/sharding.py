@@ -132,8 +132,8 @@ class TreeShardedEngine:
         fd = {"GTR": 8, "HKY": 4}.get(spec.substitution, 0) if substitution_gradient else 0
         if fd:
             keys.append(("substitution_model", fd))
-        if self.engine.category_count > 1:
-            keys.append(("site_model", 1))
+        if self.engine.category_count > 1 or self.engine.invariant:
+            keys.append(("site_model", self.engine.site_gradient_size))
         return keys
 
 
@@ -222,6 +222,41 @@ def finish_gradients_analytic(specification, taxon_count, trees, rooted, params,
                           {k: v[t].copy() for k, v in buffers.items() if k != "log_likelihood"}) for t in range(T)]
 
 
+def finish_gradients_invariant(specification, taxon_count, trees, rooted, params, log_likelihoods,
+                               branch_gradients, rate_gradients, substitution_sums, invariant_sums, category_count,
+                               site_gradient_size):
+    """sbnb_finish_gradients_invariant: raw (already reduced) sums of a +I model, among them the
+    [T][5] invariant sums (and, if not None, the [T][20] substitution sums) -> PhyloGradients whose
+    "site_model" row ends with d logL / d proportion invariant.  Host only."""
+    lib = _capi.load()
+    T, n = trees.tree_count, taxon_count
+    size = {"GTR": 8, "HKY": 4}.get(specification.substitution, 0) if substitution_sums is not None else 0
+    buffers = {"log_likelihood": np.zeros(T)}
+    if rooted:
+        buffers["ratios_root_height"] = np.zeros((T, n - 1))
+        buffers["clock_model"] = np.zeros((T, trees.rate_count))
+    else:
+        buffers["branch_lengths"] = np.zeros((T, 2 * n - 1))
+    if size:
+        buffers["substitution_model"] = np.zeros((T, size))
+    buffers["site_model"] = np.zeros((T, site_gradient_size))
+    out = _capi.GradientOutStruct()
+    for key, value in buffers.items():
+        setattr(out, key, _capi.as_double_ptr(value))
+    struct = trees.as_struct()
+    as_array = lambda a: None if a is None else np.ascontiguousarray(a, dtype=np.float64)
+    params, log_likelihoods, branch_gradients = as_array(params), as_array(log_likelihoods), as_array(branch_gradients)
+    rate_gradients = as_array(rate_gradients) if category_count > 1 else None
+    substitution_sums, invariant_sums = as_array(substitution_sums), as_array(invariant_sums)
+    _capi.check(lib.sbnb_finish_gradients_invariant(
+        specification.substitution.encode(), specification.site.encode(), specification.clock.encode(), n,
+        ctypes.byref(struct), int(rooted), _capi.as_double_ptr(params), _capi.as_double_ptr(log_likelihoods),
+        _capi.as_double_ptr(branch_gradients), _capi.as_double_ptr(rate_gradients),
+        _capi.as_double_ptr(substitution_sums), _capi.as_double_ptr(invariant_sums), ctypes.byref(out)))
+    return [PhyloGradient(float(buffers["log_likelihood"][t]),
+                          {k: v[t].copy() for k, v in buffers.items() if k != "log_likelihood"}) for t in range(T)]
+
+
 def finish_log_likelihoods_rooted(taxon_count, trees, log_likelihoods):
     """sbnb_finish_log_likelihoods_rooted: + log-det Jacobian (fat_beagle.cpp:82-94), in place."""
     struct = trees.as_struct()
@@ -248,10 +283,11 @@ class PatternShardedEngine:
             if self.world > 1:
                 self.engine.set_pattern_range(self.begin, self.end)
 
-    def _reduce(self, staged, arrays_wanted, substitution_sums=False):
+    def _reduce(self, staged, arrays_wanted, substitution_sums=False, invariant_sums=False):
         """All-reduce of the raw result arrays of a finished run, then fetch
         (arrays_wanted: 1 = log-likelihoods, 3 = + edge and rate derivatives;
-        substitution_sums: + the [T][20] sums of the analytic substitution gradient)."""
+        substitution_sums: + the [T][20] sums of the analytic substitution gradient;
+        invariant_sums: + the [T][5] sums of a +I model, which follow them on the device)."""
         lib = _capi.load()
         if self.world > 1 and self.backend == "nccl":
             import torch
@@ -261,7 +297,10 @@ class PatternShardedEngine:
             # [evaluations] log-likelihoods, [T x (2n-1)] edge derivatives and, with more than
             # one rate category, [T x (2n-1)] rate derivatives -- one collective.
             T, N = staged.tree_count, staged.node_count
-            if substitution_sums:
+            if invariant_sums:
+                count = lib.sbnb_batch_evaluation_count(staged._handle) + 2 * T * N + \
+                    (_capi.SUBSTITUTION_SUMS + _capi.INVARIANT_SUMS) * T
+            elif substitution_sums:
                 count = lib.sbnb_batch_evaluation_count(staged._handle) + 2 * T * N + _capi.SUBSTITUTION_SUMS * T
             elif arrays_wanted > 1:
                 count = lib.sbnb_batch_evaluation_count(staged._handle) + (2 if pointers[2].value else 1) * T * N
@@ -273,11 +312,15 @@ class PatternShardedEngine:
                 _dist().all_reduce(view, op=_dist().ReduceOp.SUM)
             stream.synchronize()
             result = staged.fetch(gradients=arrays_wanted > 1)
-            return (*result, staged.fetch_substitution_sums()) if substitution_sums else result
+            if substitution_sums:
+                result = (*result, staged.fetch_substitution_sums())
+            return (*result, staged.fetch_invariant_sums()) if invariant_sums else result
         result = staged.fetch(gradients=arrays_wanted > 1)
         arrays = list(result) if arrays_wanted > 1 else [result]
         if substitution_sums:
             arrays.append(staged.fetch_substitution_sums())
+        if invariant_sums:
+            arrays.append(staged.fetch_invariant_sums())
         all_reduce_sum_host(*arrays)
         return tuple(arrays) if arrays_wanted > 1 else arrays[0]
 
@@ -296,6 +339,17 @@ class PatternShardedEngine:
         fd = wanted and not analytic
         staged = self.engine.stage(trees, params, rooted=rooted, substitution_fd=fd, substitution_analytic=analytic)
         staged.run(_capi.MODE_BRANCH_GRADIENT, rescaling)
+        if self.engine.invariant:
+            if fd:
+                staged.close()
+                raise RuntimeError("A +I site model takes the analytic substitution gradient across pattern shards.")
+            arrays = self._reduce(staged, 3, substitution_sums=analytic, invariant_sums=True)
+            staged.close()
+            logl, grad, rgrad = arrays[:3]
+            return finish_gradients_invariant(self.specification, self.engine.taxon_count, trees, rooted,
+                                              self.engine._params(params, trees.tree_count), logl, grad, rgrad,
+                                              arrays[3] if analytic else None, arrays[-1], self.engine.category_count,
+                                              self.engine.site_gradient_size)
         if analytic:
             logl, grad, rgrad, sums = self._reduce(staged, 3, substitution_sums=True)
             staged.close()
@@ -309,4 +363,5 @@ class PatternShardedEngine:
 
 
 __all__ = ["TreeShardedEngine", "PatternShardedEngine", "shard_range", "pattern_range", "all_reduce_sum_host",
-           "all_gather_rows", "finish_gradients", "finish_gradients_analytic", "finish_log_likelihoods_rooted", "gather_gradients", "TreeBatch"]
+           "all_gather_rows", "finish_gradients", "finish_gradients_analytic", "finish_gradients_invariant",
+           "finish_log_likelihoods_rooted", "gather_gradients", "TreeBatch"]
