@@ -125,7 +125,12 @@ int sbnb_gp_process_operations(sbnb_gp_engine* engine, const int32_t* program, i
  *     (GPEngine::ProcessOperations, gp_engine.cpp:167-171);
  *   - word 0 of the first record of a run of mutually independent records of one kind
  *     carries the run length in bits 8..15 (the interpreter issues their loads together);
- *     the opcode is word 0 & 0xff.
+ *     the opcode is word 0 & 0xff;
+ *   - bit 16 of word 0 of an increment (bit 16 + u for source u of a kind-10 record) marks a rootward
+ *     source: a PLV that carries the stationary distribution (SetToStationaryDistribution, and every
+ *     PLV computed from one), which evolves as P(t)^T r -- P(t) is not symmetric unless the
+ *     frequencies are equal.  The directions follow the program in its order, starting from no
+ *     rootward PLV (sbnb_gp_process_operations starts from what the engine's earlier programs left).
  * out must hold word_count words; *out_word_count (<= word_count) of them are written.
  */
 int sbnb_gp_schedule_program(int32_t plv_count, int32_t gpcsp_count, const int32_t* program,
@@ -186,6 +191,12 @@ int sbnb_gp_get_plv(sbnb_gp_engine* engine, int32_t plv_idx, double* out);
 int sbnb_gp_get_rescaling_counts(sbnb_gp_engine* engine, int32_t* out);
 int64_t sbnb_gp_launch_count(const sbnb_gp_engine* engine);
 double sbnb_gp_last_kernel_ms(const sbnb_gp_engine* engine);
+/* The interpreter's launch plan for the current shape (patterns x categories, PLV and GPCSP
+ * counts), for tests that claim a regime: out[0] threads per CTA, out[1] CTAs, out[2] 1 when a
+ * multi-CTA grid runs as one thread-block cluster, out[3] 1 when the transition matrices and q
+ * live in shared memory (0: global memory), out[4] 1 when the per-warp rescaling counts live in
+ * shared memory (0: global memory), out[5] doubles of UpdateSBNProbabilities scratch. */
+int sbnb_gp_debug_launch_plan(const sbnb_gp_engine* engine, int32_t* out);
 
 #ifdef __cplusplus
 }

@@ -157,6 +157,7 @@ SIGNATURES.update({
     "sbnb_gp_get_rescaling_counts": (_c.c_int, [_c.c_void_p, _P(_c.c_int32)]),
     "sbnb_gp_launch_count": (_c.c_int64, [_c.c_void_p]),
     "sbnb_gp_last_kernel_ms": (_c.c_double, [_c.c_void_p]),
+    "sbnb_gp_debug_launch_plan": (_c.c_int, [_c.c_void_p, _P(_c.c_int32)]),
 })
 
 MODE_LOG_LIKELIHOOD = 0

@@ -136,6 +136,19 @@ __device__ __forceinline__ void TransitionMatrix(const GpParams& p, double t, bo
     }
 }
 
+// M <- M^T: a rootward PLV r evolves along an edge as P(t)^T r (r holds the stationary
+// distribution, and P(t) is not symmetric unless the frequencies are equal).
+__device__ __forceinline__ void TransposeInPlace(double (&m)[16]) {
+#pragma unroll
+  for (int i = 0; i < 4; i++)
+#pragma unroll
+    for (int j = i + 1; j < 4; j++) {
+      const double x = m[i * 4 + j];
+      m[i * 4 + j] = m[j * 4 + i];
+      m[j * 4 + i] = x;
+    }
+}
+
 // a^T M b
 __device__ __forceinline__ double Bilinear(const double (&a)[4], const double (&m)[16],
                                            const double (&b)[4]) {
@@ -184,6 +197,11 @@ constexpr int kGpClusterBlocks = 8;  // a grid of at most this many CTAs is laun
 constexpr int kGpMaxCategories = 8;
 constexpr int kGpChain = 4;                        // sources of one fused accumulation
 constexpr int kGpFlag = 1 << 30;                   // word 0: ZeroPLV clears the count only / an accumulation starts fresh
+// Word 0 of an increment (bit 16) or of source u of a fused accumulation (bit 16 + u): the source is a
+// rootward PLV -- it carries the stationary distribution (SetToStationaryDistribution, and every PLV
+// computed from one) -- and evolves as P(t)^T r.  P(t) is not symmetric unless the frequencies are
+// equal, so the direction matters beyond JC69.  The host finds the directions (CompileProgram).
+constexpr int kGpRootwardSource = 1 << 16;
 constexpr int SBNB_GP_INTERNAL_EVOLVE_SUM = 10;    // dest, n, (gpcsp, src) x n: produced by CompileProgram only
 #ifndef SBNB_GP_BATCH_OPS
 #define SBNB_GP_BATCH_OPS 2
@@ -539,6 +557,7 @@ __device__ __forceinline__ void GpInterpretBody(const GpParams& p, const GpSmemP
         int gpcsp[kGpBatch];
         double factor[kGpBatch];
         bool fresh[kGpBatch];  // the sum starts from 0: dest is not loaded
+        bool transpose[kGpBatch];  // a rootward source: P^T
         int faulty = -1;  // (no return inside the unrolled loops: they must stay unrolled for the arrays to be registers)
 #pragma unroll
         for (int u = 0; u < kGpBatch; u++) {
@@ -552,6 +571,7 @@ __device__ __forceinline__ void GpInterpretBody(const GpParams& p, const GpSmemP
             if (difference < 0 && faulty < 0) faulty = u;
             factor[u] = q[gpcsp[u]];
             if (difference > 0) factor[u] *= pow(p.threshold, static_cast<double>(difference));
+            transpose[u] = (program[pc + 4 * u] & kGpRootwardSource) != 0;
           }
         }
         if (faulty >= 0) {
@@ -576,6 +596,7 @@ __device__ __forceinline__ void GpInterpretBody(const GpParams& p, const GpSmemP
             if (u < batch) {
               double m[16];
               load_matrix(gpcsp[u], m);
+              if (transpose[u]) TransposeInPlace(m);
 #pragma unroll
               for (int i = 0; i < 4; i++)
                 d[u][i] += factor[u] * fma(m[i * 4 + 3], s[u][3],
@@ -597,6 +618,7 @@ __device__ __forceinline__ void GpInterpretBody(const GpParams& p, const GpSmemP
         const double* src_plv[kGpChain];
         int gpcsp[kGpChain];
         double factor[kGpChain];
+        bool transpose[kGpChain];  // a rootward source: P^T
         int faulty = -1;
 #pragma unroll
         for (int u = 0; u < kGpChain; u++) {
@@ -608,6 +630,7 @@ __device__ __forceinline__ void GpInterpretBody(const GpParams& p, const GpSmemP
             if (difference < 0 && faulty < 0) faulty = u;
             factor[u] = q[gpcsp[u]];
             if (difference > 0) factor[u] *= pow(p.threshold, static_cast<double>(difference));
+            transpose[u] = (word0 & (kGpRootwardSource << u)) != 0;
           }
         }
         if (faulty >= 0) {
@@ -625,6 +648,7 @@ __device__ __forceinline__ void GpInterpretBody(const GpParams& p, const GpSmemP
             if (u < sources) {
               double m[16];
               load_matrix(gpcsp[u], m);
+              if (transpose[u]) TransposeInPlace(m);
 #pragma unroll
               for (int i = 0; i < 4; i++)
                 d[i] += factor[u] * fma(m[i * 4 + 3], s[u][3], fma(m[i * 4 + 2], s[u][2], fma(m[i * 4 + 1], s[u][1], m[i * 4] * s[u][0])));
@@ -1213,6 +1237,7 @@ namespace {
 // same arithmetic in the same order as in the reference's sequence: bit-identical results.
 struct CompiledProgram {
   std::vector<int32_t> source;  // the caller's words (cache key)
+  uint64_t rootward_generation = 0;  // (of the engine's direction flags it was compiled against)
   std::vector<int32_t> words;   // what the device runs
   std::vector<std::pair<int32_t, int32_t>> origin;  // (word offset in `words`, word offset in `source`) per op
   DeviceArray<int32_t> device;
@@ -1237,6 +1262,10 @@ struct sbnb_gp_engine {
   std::vector<uint8_t> host_tips;  // [taxon][pattern], for re-initialising the PLVs when the site model changes
   bool tip_masks = false;          // host_tips are nucleotide masks (SBNB_TIPS_NUCLEOTIDE_MASKS), not states
   DeviceArray<int32_t> counts, program, status, tips;
+  // [plv] 1: a rootward PLV (kGpRootwardSource), as the programs run so far left it; a compiled
+  // program is valid for the generation of these flags it was compiled against
+  std::vector<uint8_t> rootward;
+  uint64_t rootward_generation = 0;
   // programs seen before (the reference regenerates the same few schedules call after call)
   std::vector<std::unique_ptr<CompiledProgram>> compiled;
   uint64_t program_clock = 0;
@@ -1255,7 +1284,7 @@ struct sbnb_gp_engine {
 namespace {
 
 void CompileProgram(int32_t plv_count, int32_t gpcsp_count, const int32_t* program, int64_t word_count,
-                    CompiledProgram* out);
+                    std::vector<uint8_t>* rootward, CompiledProgram* out);
 void SetCategories(sbnb_gp_engine* e, int categories, const double* rates, const double* proportions);
 
 void Bind(sbnb_gp_engine* e) { SBNB_CUDA(cudaSetDevice(e->device)); }
@@ -1486,6 +1515,8 @@ void SetCategories(sbnb_gp_engine* e, int categories, const double* rates, const
   SBNB_CUDA(cudaMemsetAsync(e->counts.get(), 0, count_copies * e->plv_count * sizeof(int32_t), e->stream));
   e->exchange.Reserve(static_cast<size_t>(2) * e->blocks * 2 * kGpReduceValues);  // 8-byte words
   e->matrix_cache.Reserve(gpcsps * 16 * categories);
+  e->rootward.assign(e->plv_count, 0);
+  e->rootward_generation++;
   SBNB_CUDA(cudaStreamSynchronize(e->stream));
   GpParams& p = e->params;
   p.pattern_count = P;
@@ -1505,7 +1536,7 @@ void SetCategories(sbnb_gp_engine* e, int categories, const double* rates, const
 }
 
 void CompileProgram(int32_t plv_count, int32_t gpcsp_count, const int32_t* program, int64_t word_count,
-                    CompiledProgram* out) {
+                    std::vector<uint8_t>* rootward, CompiledProgram* out) {
   // ---- pass 1: the caller's records; runs of IncrementWithWeightedEvolvedPLV into one PLV
   // (the reference emits a node's increments side by side, gp_dag.cpp:264-290) become ONE
   // record -- SBNB_GP_INTERNAL_EVOLVE_SUM: dest, n, (gpcsp, src) x n, at most kGpChain sources --
@@ -1537,6 +1568,7 @@ void CompileProgram(int32_t plv_count, int32_t gpcsp_count, const int32_t* progr
         case SBNB_GP_SET_TO_STATIONARY:
           size = 3;
           touch(w[1]);
+          (*rootward)[w[1]] = 1;
           break;
         case SBNB_GP_INCREMENT_WITH_EVOLVED: {
           size = 4;
@@ -1560,11 +1592,17 @@ void CompileProgram(int32_t plv_count, int32_t gpcsp_count, const int32_t* progr
           if (fresh) ops[zeroed_by[dest]].words[0] |= kGpFlag;  // that ZeroPLV: rescaling count only
           touch(dest);
           for (const auto& source : sources) touch(source.second);
+          int32_t directions = 0;
+          for (size_t u = 0; u < sources.size(); u++)
+            if ((*rootward)[sources[u].second]) directions |= kGpRootwardSource << u;
+          if (directions) (*rootward)[dest] = 1;
           if (sources.size() == 1) {
-            op.words = {SBNB_GP_INCREMENT_WITH_EVOLVED | (fresh ? kGpFlag : 0), dest, sources[0].first, sources[0].second};
+            op.words = {SBNB_GP_INCREMENT_WITH_EVOLVED | (fresh ? kGpFlag : 0) | directions, dest, sources[0].first,
+                        sources[0].second};
           } else {
             op.opcode = SBNB_GP_INTERNAL_EVOLVE_SUM;
-            op.words = {SBNB_GP_INTERNAL_EVOLVE_SUM | (fresh ? kGpFlag : 0), dest, static_cast<int32_t>(sources.size())};
+            op.words = {SBNB_GP_INTERNAL_EVOLVE_SUM | (fresh ? kGpFlag : 0) | directions, dest,
+                        static_cast<int32_t>(sources.size())};
             for (const auto& source : sources) op.words.insert(op.words.end(), {source.first, source.second});
           }
           size = static_cast<int32_t>(next - pc);
@@ -1573,6 +1611,7 @@ void CompileProgram(int32_t plv_count, int32_t gpcsp_count, const int32_t* progr
         case SBNB_GP_MULTIPLY:
           size = 4;
           touch(w[1]), touch(w[2]), touch(w[3]);
+          if ((*rootward)[w[2]] || (*rootward)[w[3]]) (*rootward)[w[1]] = 1;
           break;
         case SBNB_GP_LIKELIHOOD:
         case SBNB_GP_INCREMENT_MARGINAL:
@@ -1595,7 +1634,13 @@ void CompileProgram(int32_t plv_count, int32_t gpcsp_count, const int32_t* progr
         default:
           Fail(SBNB_ERR_INVALID_ARGUMENT, "Unknown GP opcode " + std::to_string(opcode) + ".");
       }
-      if (op.words.empty()) op.words.assign(w, w + size);
+      if (op.words.empty()) {
+        op.words.assign(w, w + size);
+        if (opcode == SBNB_GP_INCREMENT_WITH_EVOLVED && (*rootward)[w[3]]) {  // (not fused)
+          op.words[0] |= kGpRootwardSource;
+          (*rootward)[w[1]] = 1;
+        }
+      }
       ops.push_back(std::move(op));
       if (opcode == SBNB_GP_ZERO_PLV && fusing) zeroed_by[w[1]] = static_cast<int32_t>(ops.size()) - 1;
       if (opcode == SBNB_GP_ZERO_PLV && !fusing) touch(w[1]);
@@ -1838,6 +1883,13 @@ int sbnb_gp_process_operations(sbnb_gp_engine* e, const int32_t* program, int64_
       if (candidate->source.size() == static_cast<size_t>(word_count) &&
           std::memcmp(candidate->source.data(), program, word_count * sizeof(int32_t)) == 0)
         compiled = candidate.get();
+    if (compiled != nullptr && compiled->rootward_generation != e->rootward_generation) {
+      // compiled against direction flags that have grown since: compile it again
+      SBNB_CUDA(cudaStreamSynchronize(e->stream));
+      e->compiled.erase(std::find_if(e->compiled.begin(), e->compiled.end(),
+                                     [&](const auto& c) { return c.get() == compiled; }));
+      compiled = nullptr;
+    }
     if (compiled == nullptr) {
       ValidateProgram(GpShape{e->plv_count, e->gpcsp_count}, program, word_count);
       if (e->compiled.size() >= kGpProgramCacheSize) {
@@ -1848,7 +1900,14 @@ int sbnb_gp_process_operations(sbnb_gp_engine* e, const int32_t* program, int64_
       }
       e->compiled.push_back(std::make_unique<CompiledProgram>());
       compiled = e->compiled.back().get();
-      CompileProgram(e->plv_count, e->gpcsp_count, program, word_count, compiled);
+      const std::vector<uint8_t> before = e->rootward;
+      CompileProgram(e->plv_count, e->gpcsp_count, program, word_count, &e->rootward, compiled);
+      compiled->rootward_generation = e->rootward_generation;
+      if (e->rootward != before) {
+        // (the program's own records read the flags as they were when they ran; run again, from the
+        //  grown flags, it is compiled again)
+        e->rootward_generation++;
+      }
       compiled->device.Upload(compiled->words.data(), compiled->words.size(), e->stream);
     }
     compiled->last_used = ++e->program_clock;
@@ -1967,7 +2026,8 @@ int sbnb_gp_schedule_program(int32_t plv_count, int32_t gpcsp_count, const int32
     Require(out != nullptr || word_count == 0, "NULL output.");
     ValidateProgram(GpShape{plv_count, gpcsp_count}, program, word_count);
     CompiledProgram compiled;
-    CompileProgram(plv_count, gpcsp_count, program, word_count, &compiled);
+    std::vector<uint8_t> rootward(plv_count, 0);  // (a program on PLVs no earlier program has written)
+    CompileProgram(plv_count, gpcsp_count, program, word_count, &rootward, &compiled);
     Require(static_cast<int64_t>(compiled.words.size()) <= word_count, "The schedule outgrew the program.");
     std::copy(compiled.words.begin(), compiled.words.end(), out);
     if (out_word_count) *out_word_count = static_cast<int64_t>(compiled.words.size());
@@ -2178,5 +2238,17 @@ int sbnb_gp_get_rescaling_counts(sbnb_gp_engine* e, int32_t* out) {
 
 int64_t sbnb_gp_launch_count(const sbnb_gp_engine* e) { return e ? e->launch_count : -1; }
 double sbnb_gp_last_kernel_ms(const sbnb_gp_engine* e) { return e ? e->last_kernel_ms : -1.0; }
+
+int sbnb_gp_debug_launch_plan(const sbnb_gp_engine* e, int32_t* out) {
+  return Guard([&] {
+    Require(e && out, "NULL argument.");
+    out[0] = e->threads;
+    out[1] = e->blocks;
+    out[2] = e->blocks > 1 && e->blocks <= kGpClusterBlocks && !e->no_cluster ? 1 : 0;
+    out[3] = e->plan.matrices;
+    out[4] = e->plan.counts;
+    out[5] = e->plan.scratch;
+  });
+}
 
 }  // extern "C"

@@ -256,6 +256,15 @@ class GPEngine:
         return out
 
     @property
+    def launch_plan(self):
+        """The interpreter's launch plan (sbnb_gp_debug_launch_plan): threads per CTA, CTAs, whether the
+        grid is one cluster, and whether matrices / rescaling counts sit in shared memory."""
+        out = np.zeros(6, dtype=np.int32)
+        _capi.check(self._lib.sbnb_gp_debug_launch_plan(self._handle, _capi.as_int32_ptr(out)))
+        return {"threads": int(out[0]), "blocks": int(out[1]), "cluster": bool(out[2]),
+                "shared_matrices": bool(out[3]), "shared_counts": bool(out[4]), "scratch": int(out[5])}
+
+    @property
     def launch_count(self):
         return int(self._lib.sbnb_gp_launch_count(self._handle))
 
