@@ -43,7 +43,9 @@ extern "C" {
  * out_weights: capacity site_count doubles; the multiplicity of each pattern.
  * out_device_ms: if not NULL, the device time of the kernels (CUDA events).
  * A character outside the symbol table fails with the reference's message
- * "Symbol 'c' not known." (site_pattern.cpp:47-55).
+ * "Symbol 'c' not known." (site_pattern.cpp:47-55), naming the first such
+ * character in (taxon, site) order; a byte outside printable ASCII (0x20-0x7e)
+ * is written as \xHH.
  */
 int sbnb_compress_site_patterns(int32_t taxon_count, int64_t site_count, const char* sequences,
                                 int32_t device, uint8_t* out_patterns, double* out_weights,

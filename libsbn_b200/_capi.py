@@ -200,7 +200,8 @@ def load():
 def check(code):
     if code != 0:
         message = load().sbnb_last_error()
-        raise SbnbError(code, message.decode() if message else f"libsbn_b200 error {code}")
+        # (backslashreplace: no message byte can turn the SbnbError into a UnicodeDecodeError)
+        raise SbnbError(code, message.decode(errors="backslashreplace") if message else f"libsbn_b200 error {code}")
 
 
 def as_double_ptr(array):

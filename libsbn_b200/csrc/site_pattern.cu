@@ -119,12 +119,14 @@ __device__ __forceinline__ uint32_t HashStep(uint32_t h, uint32_t word, uint32_t
   return __funnelshift_l(h, h, r2) * m + add;
 }
 
-// status[0] = 1 + an unknown character seen (0 = none); status[1] = collision flag.
+// *unknown = the least position t * site_count + site of an unknown character (all ones = none),
+// so the report names the first one in (taxon, site) order whatever the timing.
 // MASKS: the table holds nucleotide masks 1..15, and an unknown character hashes as 0.
 template <bool MASKS>
 __global__ void __launch_bounds__(kHashThreads) HashKernel(
     const uint8_t* __restrict__ sequences, uint64_t* __restrict__ keys, int32_t taxon_count, int64_t site_count,
-    int64_t pitch, uint64_t seed, uint64_t key_mask, const SymbolTable table, int32_t* __restrict__ status) {
+    int64_t pitch, uint64_t seed, uint64_t key_mask, const SymbolTable table,
+    unsigned long long* __restrict__ unknown) {
   // character -> its symbol as a 4-bit field already in the place of taxon i of a group of 8
   // (an unknown character: 0xf, the only value with bit 3 set; with MASKS, 0, the only zero field)
   __shared__ uint32_t shifted[8][256];
@@ -180,12 +182,12 @@ __global__ void __launch_bounds__(kHashThreads) HashKernel(
     }
   }
   if (seen & 0x88888888u) {
-    // rare: find the character for the error message (padding sites hold 'A')
+    // rare: the thread's first unknown character in (taxon, site) order (padding sites hold 'A')
     for (int t = 0; t < taxon_count; t++) {
       for (int k = 0; k < kSitesPerThread; k++) {
         const uint8_t c = column[static_cast<int64_t>(t) * pitch + k];
         if (table.map[c] == kUnknownSymbol && site0 + k < site_count) {
-          atomicCAS(&status[0], 0, 1 + static_cast<int>(c));
+          atomicMin(unknown, static_cast<unsigned long long>(t * site_count + site0 + k));
           t = taxon_count;
           break;
         }
@@ -370,7 +372,7 @@ __global__ void __launch_bounds__(256) TileKernel(const uint8_t* __restrict__ se
                                                   const uint32_t* __restrict__ table_column,
                                                   uint8_t* __restrict__ columns, int32_t taxon_count,
                                                   int64_t site_count, int64_t pitch, int64_t column_pitch,
-                                                  const SymbolTable table, int32_t* __restrict__ status) {
+                                                  const SymbolTable table, int32_t* __restrict__ collided) {
   constexpr int kSiteWords = kTileTaxa / 4 + 1;  // 17: the sites of a warp's store fall into 32 banks
   __shared__ uint8_t map[256];
   __shared__ uint32_t column_of[kTileSites];
@@ -418,7 +420,19 @@ __global__ void __launch_bounds__(256) TileKernel(const uint8_t* __restrict__ se
       }
     }
   }
-  if (VERIFY && difference != 0) status[1] = 1;
+  if (VERIFY && difference != 0) *collided = 1;
+}
+
+// "Symbol 'c' not known." (SymbolTableAt, site_pattern.cpp:47-55), with a byte outside printable
+// ASCII written as \xHH so that the message stays valid text.
+std::string UnknownSymbolMessage(uint8_t c) {
+  char symbol[8];
+  if (c >= 0x20 && c <= 0x7e) {
+    std::snprintf(symbol, sizeof(symbol), "%c", c);
+  } else {
+    std::snprintf(symbol, sizeof(symbol), "\\x%02x", c);
+  }
+  return std::string("Symbol '") + symbol + "' not known.";
 }
 
 void Compress(int32_t n, int64_t S, const char* sequences, bool masks, int32_t device, uint8_t* out_patterns,
@@ -457,7 +471,7 @@ void Compress(int32_t n, int64_t S, const char* sequences, bool masks, int32_t d
   DeviceArray<unsigned long long> d_table_keys, d_total;
   DeviceArray<uint32_t> d_table_first, d_table_count, d_table_pattern, d_table_column, d_slot_of, d_flags, d_index,
       d_block_sums, d_column_counter;
-  DeviceArray<int32_t> d_status;
+  DeviceArray<int32_t> d_collided;
   DeviceArray<double> d_weights;
   d_sequences.Reserve(static_cast<size_t>(n) * pitch);
   d_keys.Reserve(S);
@@ -476,8 +490,8 @@ void Compress(int32_t n, int64_t S, const char* sequences, bool masks, int32_t d
   d_columns.Reserve(static_cast<size_t>(S / 2 + 1) * column_pitch);
   SBNB_CUDA(cudaMemset(d_flags.get(), 0, static_cast<size_t>(pitch) * sizeof(uint32_t)));
   d_block_sums.Reserve(scan_blocks);
-  d_total.Reserve(1);
-  d_status.Reserve(2);
+  d_total.Reserve(2);  // the pattern count, then the position of the first unknown character
+  d_collided.Reserve(1);
   d_weights.Reserve(pitch);
   d_patterns.Reserve(static_cast<size_t>(n) * pitch);
   stage("device allocations");
@@ -521,7 +535,8 @@ void Compress(int32_t n, int64_t S, const char* sequences, bool masks, int32_t d
   double device_ms = 0.0;
   bool done = false;
   for (uint64_t seed = 0; seed < 4 && !done; seed++) {
-    SBNB_CUDA(cudaMemset(d_status.get(), 0, 2 * sizeof(int32_t)));
+    SBNB_CUDA(cudaMemset(d_total.get() + 1, 0xff, sizeof(unsigned long long)));
+    SBNB_CUDA(cudaMemset(d_collided.get(), 0, sizeof(int32_t)));
     SBNB_CUDA(cudaMemset(d_column_counter.get(), 0, sizeof(uint32_t)));
     SBNB_CUDA(cudaMemset(d_table_keys.get(), 0xff, static_cast<size_t>(table_size) * sizeof(uint64_t)));
     SBNB_CUDA(cudaMemset(d_table_first.get(), 0xff, static_cast<size_t>(table_size) * sizeof(uint32_t)));
@@ -530,7 +545,7 @@ void Compress(int32_t n, int64_t S, const char* sequences, bool masks, int32_t d
     const int64_t groups = pitch / kSitesPerThread;
     (masks ? HashKernel<true> : HashKernel<false>)<<<static_cast<int>((groups + kHashThreads - 1) / kHashThreads),
                                                      kHashThreads>>>(
-        d_sequences.get(), d_keys.get(), n, S, pitch, seed * 0x9e3779b97f4a7c15ull, key_mask, table, d_status.get());
+        d_sequences.get(), d_keys.get(), n, S, pitch, seed * 0x9e3779b97f4a7c15ull, key_mask, table, d_total.get() + 1);
     InsertKernel<<<site_blocks, 256>>>(d_keys.get(), d_table_keys.get(), d_table_first.get(),
                                        d_table_count.get(), d_slot_of.get(), S, table_size - 1);
     FlagKernel<<<site_blocks, 256>>>(d_slot_of.get(), d_table_first.get(), d_flags.get(), S);
@@ -547,27 +562,24 @@ void Compress(int32_t n, int64_t S, const char* sequences, bool masks, int32_t d
     // pattern's column byte for byte
     TileKernel<false><<<static_cast<int>(pitch / kTileSites), 256>>>(d_sequences.get(), d_slot_of.get(), d_flags.get(),
                                                                      d_table_column.get(), d_columns.get(), n, S, pitch,
-                                                                     column_pitch, table, d_status.get());
+                                                                     column_pitch, table, d_collided.get());
     TileKernel<true><<<static_cast<int>(pitch / kTileSites), 256>>>(d_sequences.get(), d_slot_of.get(), d_flags.get(),
                                                                     d_table_column.get(), d_columns.get(), n, S, pitch,
-                                                                    column_pitch, table, d_status.get());
+                                                                    column_pitch, table, d_collided.get());
     SBNB_CUDA(cudaEventRecord(end));
     SBNB_CUDA(cudaGetLastError());
     SBNB_CUDA(cudaEventSynchronize(end));
     float ms = 0.f;
     SBNB_CUDA(cudaEventElapsedTime(&ms, begin, end));
     device_ms = ms;
-    int32_t status[2];
-    unsigned long long total = 0;
-    SBNB_CUDA(cudaMemcpy(status, d_status.get(), sizeof(status), cudaMemcpyDeviceToHost));
-    SBNB_CUDA(cudaMemcpy(&total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost));
-    if (status[0] != 0) {
-      // SymbolTableAt (site_pattern.cpp:47-55)
-      Fail(SBNB_ERR_INVALID_ARGUMENT,
-           std::string("Symbol '") + static_cast<char>(status[0] - 1) + "' not known.");
-    }
-    if (status[1] != 0) continue;  // two different columns shared a 64-bit key: rehash
-    pattern_count = static_cast<int64_t>(total);
+    int32_t collided = 0;
+    unsigned long long total[2] = {0, 0};
+    SBNB_CUDA(cudaMemcpy(&collided, d_collided.get(), sizeof(collided), cudaMemcpyDeviceToHost));
+    SBNB_CUDA(cudaMemcpy(total, d_total.get(), sizeof(total), cudaMemcpyDeviceToHost));
+    if (total[1] != ~0ull)
+      Fail(SBNB_ERR_INVALID_ARGUMENT, UnknownSymbolMessage(static_cast<uint8_t>(sequences[total[1]])));
+    if (collided != 0) continue;  // two different columns shared a 64-bit key: rehash
+    pattern_count = static_cast<int64_t>(total[0]);
     done = true;
   }
   if (!done) Fail(SBNB_ERR_CUDA, "Site pattern hashing collided under four seeds.");

@@ -20,13 +20,18 @@ def symbol_table():
     return table
 
 
+def symbol_text(byte):
+    """A character as the error message writes it: printable ASCII verbatim, other bytes as \\xHH."""
+    return chr(byte) if 0x20 <= byte <= 0x7e else f"\\x{int(byte):02x}"
+
+
 def compress(sequences):
     """sequences: equal-length strings in leaf-id order -> (patterns uint8 [taxon][pattern], weights)."""
     rows = np.array([np.frombuffer(s.encode() if isinstance(s, str) else s, dtype=np.uint8) for s in sequences])
     symbols = symbol_table()[rows]
     if (symbols == 255).any():
         t, k = np.argwhere(symbols == 255)[np.lexsort(np.argwhere(symbols == 255).T[::-1])][0]
-        raise RuntimeError(f"Symbol '{chr(rows[t, k])}' not known.")
+        raise RuntimeError(f"Symbol '{symbol_text(rows[t, k])}' not known.")
     if rows.shape[1] == 0:
         return np.zeros((rows.shape[0], 0), np.uint8), np.zeros(0)
     _, first, counts = np.unique(symbols, axis=1, return_index=True, return_counts=True)
