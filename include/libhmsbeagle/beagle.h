@@ -4,15 +4,18 @@
  *
  * BEAGLE (beagle-dev/beagle-lib, branch hmc-clock, unpinned: reference
  * README.md:16-19, SConstruct:187-197) is a third-party dependency that is NOT
- * vendored in the reference tree.  This header declares exactly the 17 C entry
- * points, 2 structs and the flag / return-code enums that the reference calls
- * (all call sites: src/fat_beagle.cpp; flag names:
- * src/beagle_flag_names.hpp:22-54; python enum: src/pylibsbn.cpp:448-475), so
- * that the UNMODIFIED reference host code compiles against it.  Two libraries
+ * vendored in the reference tree.  This header declares the 17 C entry points,
+ * 2 structs and the flag / return-code enums that the reference calls (all call
+ * sites: src/fat_beagle.cpp; flag names: src/beagle_flag_names.hpp:22-54; python
+ * enum: src/pylibsbn.cpp:448-475), so that the UNMODIFIED reference host code
+ * compiles against it, plus one standard BEAGLE call the reference does not make,
+ * beagleGetSiteLogLikelihoods (per-pattern log-likelihoods for topology tests and
+ * model comparison).  Two libraries
  * implement this ABI:
  *   - libsbn_b200/csrc/beagle_shim.cu -> libhmsbeagle_b200.so: every call runs on
  *     the B200 (the product's compatibility path: relink, nothing else changes);
- *   - oracle/beagle_cpu.cpp: the CPU restatement used only as the test oracle.
+ *   - oracle/beagle_cpu.cpp: the CPU restatement used only as the test oracle (the 17
+ *     calls the reference makes; not beagleGetSiteLogLikelihoods).
  * The performance path is the outer boundary, include/sbn_b200.h.
  *
  * Written from the reference's call sites and the published BEAGLE API
@@ -153,6 +156,13 @@ int beagleCalculateRootLogLikelihoods(int instance, const int* bufferIndices,
                                       const int* stateFrequenciesIndices,
                                       const int* cumulativeScaleIndices, int count,
                                       double* outSumLogLikelihood);
+
+/* ---- a standard BEAGLE call the reference does not make ---------------------------------- */
+
+/* The per-pattern log-likelihoods of the most recent beagleCalculateRootLogLikelihoods on the
+ * instance (cumulative scale factors included, pattern weights not): patternCount doubles.
+ * An error before any root call.  (Declared extern, apart from the 17 calls above.) */
+extern int beagleGetSiteLogLikelihoods(int instance, double* outLogLikelihoods);
 
 #ifdef __cplusplus
 }

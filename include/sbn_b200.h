@@ -191,6 +191,25 @@ int sbnb_log_likelihoods_rooted(sbnb_engine* engine, const sbnb_tree_batch* tree
 int sbnb_unrooted_log_likelihoods_of_rooted(sbnb_engine* engine, const sbnb_tree_batch* trees,
                                             const double* params, int32_t rescaling,
                                             double* out_log_likelihoods);
+/*
+ * Site log-likelihoods: for tree t and site pattern k of the engine's pattern range,
+ * out_site[t][k] is the log site likelihood the walk adds into logL_t with weight w_k --
+ * log(site likelihood) + (power-of-two exponent) ln 2 with rescaling, log((1 - p) L_k + p I_k)
+ * with +I -- unweighted, so that sum_k w_k out_site[t][k] = logL_t up to summation order.
+ * A pattern of weight 0 gets its value too; an unrescaled site that underflows gives -inf, as
+ * its term in the sum would.  out_log_likelihoods ([T], or NULL) is bitwise what
+ * sbnb_log_likelihoods_unrooted / _rooted return for the same input.  Rooted trees: the
+ * values are for the branch lengths times the rates and exclude the log-det Jacobian, so
+ * sum_k w_k out_site[t][k] = logL_t - logdetJ_t (sbnb_finish_log_likelihoods_rooted applied
+ * to zeros gives logdetJ_t).  A device group fills the whole [T][pattern_count] matrix on
+ * either shard axis.  For RELL / KH / SH / AU topology tests and PSIS-LOO / WAIC.
+ */
+int sbnb_site_log_likelihoods_unrooted(sbnb_engine* engine, const sbnb_tree_batch* trees,
+                                       const double* params, int32_t rescaling,
+                                       double* out_log_likelihoods, double* out_site);
+int sbnb_site_log_likelihoods_rooted(sbnb_engine* engine, const sbnb_tree_batch* trees,
+                                     const double* params, int32_t rescaling,
+                                     double* out_log_likelihoods, double* out_site);
 /* Engine::Gradients(UnrootedTreeCollection) (engine.cpp:78-84). */
 int sbnb_gradients_unrooted(sbnb_engine* engine, const sbnb_tree_batch* trees,
                             const double* params, int32_t rescaling,
@@ -211,11 +230,16 @@ enum {
   SBNB_STAGE_SUBSTITUTION_FD = 2, /* also stage the 2 x (5+3) perturbed models of the
                                      finite-difference substitution gradient
                                      (fat_beagle.cpp:400-465) as extra logL-only evaluations */
-  SBNB_STAGE_SUBSTITUTION_ANALYTIC = 4 /* gradient runs also accumulate the 20 sums per tree of
+  SBNB_STAGE_SUBSTITUTION_ANALYTIC = 4, /* gradient runs also accumulate the 20 sums per tree of
                                      the analytic substitution gradient (see
                                      sbnb_engine_set_substitution_gradient); fetched with
                                      sbnb_batch_fetch_substitution_sums, they follow the rate
                                      gradients in the device result array */
+  SBNB_STAGE_SITE_LOG_LIKELIHOODS = 8 /* log-likelihood runs also write the [T][P] site
+                                     log-likelihoods (P = the engine's pattern range when
+                                     staged; T x P doubles of device memory, allocated only
+                                     with this flag); fetched with
+                                     sbnb_batch_fetch_site_log_likelihoods */
 };
 
 /* Builds the per-tree traversal programs and eigen-systems on the host and
@@ -243,6 +267,12 @@ int sbnb_batch_fetch_substitution_sums(sbnb_engine* engine, sbnb_batch* batch, d
  * Sums over site patterns: ranks that each hold a pattern range add them like the other raw
  * results (on the device they follow the substitution sums in the result array). */
 int sbnb_batch_fetch_invariant_sums(sbnb_engine* engine, sbnb_batch* batch, double* sums);
+/* The [T][P] site log-likelihoods (see sbnb_site_log_likelihoods_unrooted) of the last run of
+ * a batch staged with SBNB_STAGE_SITE_LOG_LIKELIHOODS, P = the width of the pattern range it was
+ * staged on (which a run requires unchanged).  SBNB_ERR_INVALID_ARGUMENT if the batch was staged
+ * without the flag, has not been run, or was last run in gradient mode (gradient runs do not
+ * write them). */
+int sbnb_batch_fetch_site_log_likelihoods(sbnb_engine* engine, sbnb_batch* batch, double* out);
 /* Device addresses of the raw result arrays sbnb_batch_fetch copies out
  * (fp64: [evaluation_count], [T][2n-1], [T][2n-1]), valid until the batch is
  * destroyed.  For site-pattern sharding: the ranks sum-all-reduce these in

@@ -79,6 +79,10 @@ SIGNATURES = {
                                                _c.c_int32, _P(_c.c_double)]),
     "sbnb_unrooted_log_likelihoods_of_rooted": (_c.c_int, [_c.c_void_p, _P(TreeBatchStruct),
                                                            _P(_c.c_double), _c.c_int32, _P(_c.c_double)]),
+    "sbnb_site_log_likelihoods_unrooted": (_c.c_int, [_c.c_void_p, _P(TreeBatchStruct), _P(_c.c_double),
+                                                      _c.c_int32, _P(_c.c_double), _P(_c.c_double)]),
+    "sbnb_site_log_likelihoods_rooted": (_c.c_int, [_c.c_void_p, _P(TreeBatchStruct), _P(_c.c_double),
+                                                    _c.c_int32, _P(_c.c_double), _P(_c.c_double)]),
     "sbnb_gradients_unrooted": (_c.c_int, [_c.c_void_p, _P(TreeBatchStruct), _P(_c.c_double),
                                            _c.c_int32, _P(GradientOutStruct)]),
     "sbnb_gradients_rooted": (_c.c_int, [_c.c_void_p, _P(TreeBatchStruct), _P(_c.c_double),
@@ -94,6 +98,7 @@ SIGNATURES = {
                                                   _P(TreeBatchStruct), _c.c_int32, _P(_c.c_double), _P(_c.c_double),
                                                   _P(_c.c_double), _P(_c.c_double), _P(_c.c_double),
                                                   _P(GradientOutStruct)]),
+    "sbnb_batch_fetch_site_log_likelihoods": (_c.c_int, [_c.c_void_p, _c.c_void_p, _P(_c.c_double)]),
     "sbnb_batch_fetch_invariant_sums": (_c.c_int, [_c.c_void_p, _c.c_void_p, _P(_c.c_double)]),
     "sbnb_finish_gradients_invariant": (_c.c_int, [_c.c_char_p, _c.c_char_p, _c.c_char_p, _c.c_int32,
                                                    _P(TreeBatchStruct), _c.c_int32, _P(_c.c_double), _P(_c.c_double),
@@ -165,6 +170,7 @@ MODE_BRANCH_GRADIENT = 1
 STAGE_ROOTED = 1
 STAGE_SUBSTITUTION_FD = 2
 STAGE_SUBSTITUTION_ANALYTIC = 4
+STAGE_SITE_LOG_LIKELIHOODS = 8
 SUBSTITUTION_SUMS = 20
 INVARIANT_SUMS = 5  # +I: D, then E_A..E_T (sbnb_batch_fetch_invariant_sums)
 SHARD_TREES = 0

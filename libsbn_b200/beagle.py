@@ -102,6 +102,13 @@ class Beagle:
         self.ok(self.lib.beagleCalculateRootLogLikelihoods(self.handle, root, zero, zero, cum, 1, ctypes.byref(logl)))
         return logl.value, sums, squares, per_site_values
 
+    def site_log_likelihoods(self):
+        """beagleGetSiteLogLikelihoods: [P] per-pattern log-likelihoods of the last root call
+        (cumulative scale factors included, pattern weights not)."""
+        out = np.empty(self.P)
+        self.ok(self.lib.beagleGetSiteLogLikelihoods(self.handle, out.ctypes.data_as(_D)))
+        return out
+
     def close(self):
         self.ok(self.lib.beagleFinalizeInstance(self.handle))
 

@@ -497,9 +497,11 @@ __device__ __forceinline__ double BlockSum(double value, double* smem) {
 }
 
 // beagleCalculateRootLogLikelihoods (fat_beagle.cpp:65-68, 170-173):
-//   sum_k w_k (log sum_i pi_i sum_c p_c root[c,k,i] + cumulative_k)  -> per-block partial sums
+//   sum_k w_k (log sum_i pi_i sum_c p_c root[c,k,i] + cumulative_k)  -> per-block partial sums,
+//   and every pattern's term before its weight -> site_logl (beagleGetSiteLogLikelihoods)
 __global__ void __launch_bounds__(kBlock) RootLogLikelihoodKernel(const InstanceView v, int root, int cumulative,
-                                                                 double* __restrict__ block_sums) {
+                                                                 double* __restrict__ block_sums,
+                                                                 double* __restrict__ site_logl) {
   __shared__ double smem[kBlock / 32];
   double local = 0.0;
   const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
@@ -516,6 +518,7 @@ __global__ void __launch_bounds__(kBlock) RootLogLikelihoodKernel(const Instance
     for (int i = 0; i < 4; i++) site += v.freqs[i] * over_categories[i];
     double log_site = log(site);
     if (cumulative >= 0) log_site += v.scale[static_cast<size_t>(cumulative) * v.P + k];
+    site_logl[k] = log_site;
     local += v.pattern_weights[k] * log_site;
   }
   const double total = BlockSum(local, smem);
@@ -645,6 +648,8 @@ struct Instance {
   cudaStream_t stream = nullptr;
   cudaEvent_t begin = nullptr, end = nullptr;
   DeviceBuffer<double> partials, matrix, scale, cat_weights, cat_rates, freqs, pattern_weights, staging, sums, out;
+  DeviceBuffer<double> site_logl;  // [P] of the last root call
+  bool has_site_logl = false;
   DeviceBuffer<uint8_t> compact, is_compact;
   DeviceBuffer<int32_t> indices;
   DeviceBuffer<DeviceOp> ops;
@@ -1128,9 +1133,10 @@ int beagleCalculateRootLogLikelihoods(int instance, const int* bufferIndices, co
   if (cumulative != BEAGLE_OP_NONE && (cumulative < 0 || cumulative >= inst->scalers)) return BEAGLE_ERROR_OUT_OF_RANGE;
   SHIM_CUDA(cudaSetDevice(inst->device));
   const int blocks = std::min(inst->PatternBlocks(), 256);
-  if (!inst->sums.Reserve(blocks) || !inst->out.Reserve(1)) return BEAGLE_ERROR_OUT_OF_MEMORY;
-  RootLogLikelihoodKernel<<<blocks, kBlock, 0, inst->stream>>>(inst->View(), root,
-                                                               cumulative == BEAGLE_OP_NONE ? -1 : cumulative, inst->sums.ptr);
+  if (!inst->sums.Reserve(blocks) || !inst->out.Reserve(1) || !inst->site_logl.Reserve(std::max(inst->P, 1)))
+    return BEAGLE_ERROR_OUT_OF_MEMORY;
+  RootLogLikelihoodKernel<<<blocks, kBlock, 0, inst->stream>>>(
+      inst->View(), root, cumulative == BEAGLE_OP_NONE ? -1 : cumulative, inst->sums.ptr, inst->site_logl.ptr);
   SHIM_CUDA(cudaGetLastError());
   SumBlocksKernel<<<1, 32, 0, inst->stream>>>(inst->sums.ptr, blocks, 1, 1, inst->out.ptr);
   SHIM_CUDA(cudaGetLastError());
@@ -1139,7 +1145,21 @@ int beagleCalculateRootLogLikelihoods(int instance, const int* bufferIndices, co
   SHIM_CUDA(cudaMemcpyAsync(&total, inst->out.ptr, sizeof(double), cudaMemcpyDeviceToHost, inst->stream));
   SHIM_CUDA(cudaStreamSynchronize(inst->stream));
   *outSumLogLikelihood = total;
+  inst->has_site_logl = true;
   return std::isnan(total) ? BEAGLE_ERROR_FLOATING_POINT : BEAGLE_SUCCESS;
+}
+
+// The values the last root call stored (not recomputed: the root buffer may have changed since).
+int beagleGetSiteLogLikelihoods(int instance, double* outLogLikelihoods) {
+  Instance* inst = Get(instance);
+  if (!inst) return BEAGLE_ERROR_UNINITIALIZED_INSTANCE;
+  if (!outLogLikelihoods) return BEAGLE_ERROR_OUT_OF_RANGE;
+  if (!inst->has_site_logl) return BEAGLE_ERROR_GENERAL;  // no beagleCalculateRootLogLikelihoods yet
+  SHIM_CUDA(cudaSetDevice(inst->device));
+  SHIM_CUDA(cudaMemcpyAsync(outLogLikelihoods, inst->site_logl.ptr, static_cast<size_t>(inst->P) * sizeof(double),
+                            cudaMemcpyDeviceToHost, inst->stream));
+  SHIM_CUDA(cudaStreamSynchronize(inst->stream));
+  return BEAGLE_SUCCESS;
 }
 
 // Not BEAGLE: diagnostics of this implementation (device time, ms by CUDA events, of the last

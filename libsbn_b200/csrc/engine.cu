@@ -119,6 +119,7 @@ struct sbnb_batch {
   bool with_subst = false;  // staged for the analytic substitution gradient (Phi in the pre-order blocks)
   bool rooted_finish = false;  // time-tree fields staged: gradient runs end with RootedFinishKernel
   bool invariant = false;      // +I: gradient runs also reduce the kOeInvariantSums sums per tree
+  bool with_sites = false;     // SBNB_STAGE_SITE_LOG_LIKELIHOODS: log-likelihood runs also write site_logl
   int site_width = 1;          // entries of a tree's site-model gradient (ModelSpec::SiteGradientSize)
   int rate_count = 0;
   size_t children_at = 0, rooted_fields_at = 0;
@@ -146,20 +147,22 @@ struct sbnb_batch {
   int64_t operand_stride = 0;                  // of the base trees' blocks in `operands` (last run)
   DeviceArray<double> operands;                // operand blocks of the base trees
   DeviceArray<double> logl_partial, grad_partial, rgrad_partial, subst_partial, inv_partial;
+  DeviceArray<double> site_logl;  // [T][patterns] log site likelihoods (batches staged with_sites)
   // [logl (vtree_count) | grad (T x N) | rgrad (T x N) | subst sums (T x 20) | +I sums (T x 5) | rooted finish]
   DeviceArray<double> results;
   // tiling of the last run
   int chunks = 1;
   // One-call entry points on an unchanged topology set replay the launch sequence
   // [matrices, walk(s), reduce, results -> host] as a CUDA graph (one per mode and
-  // rescaling flag), re-captured whenever a buffer it names has moved.
+  // rescaling flag; log-likelihood runs with and without the site matrix apart), re-captured
+  // whenever a buffer it names has moved.
   struct Graph {
     cudaGraphExec_t exec = nullptr;
     std::vector<uintptr_t> signature;
     int kernels = 0;
     bool warm = false;  // this very sequence has run eagerly since the programs were staged: buffers sized
   };
-  Graph graphs[2][2];
+  Graph graphs[3][2];  // [log-likelihood | gradient | log-likelihood + sites][rescaling]
   int cache_hits = 0;  // consecutive Stage() calls that found the programs on the device
   ~sbnb_batch() {
     for (auto& row : graphs)
@@ -219,9 +222,9 @@ struct LaunchPlan {
 };
 
 // Plans (and launches) TreeWalkOeKernel, whose tiles are kThreads / C * K patterns.
-template <int C, int K, bool GRAD, bool RESCALE, bool SUBST, bool AMBIG, bool INVAR>
+template <int C, int K, bool GRAD, bool RESCALE, bool SUBST, bool AMBIG, bool INVAR, bool SITES>
 LaunchPlan PlanAndLaunchOe(sbnb_engine* e, OeParams p, bool launch, int chunks_override) {
-  auto kernel = TreeWalkOeKernel<C, K, GRAD, RESCALE, SUBST, AMBIG, INVAR>;
+  auto kernel = TreeWalkOeKernel<C, K, GRAD, RESCALE, SUBST, AMBIG, INVAR, SITES>;
   // (SBNB_EXTRA_SMEM: development aid -- pads the request to lower the resident CTA count)
   const size_t smem =
       OeSmemBytes(C, K, GRAD, SUBST, AMBIG) + static_cast<size_t>(std::max(0, EnvInt("SBNB_EXTRA_SMEM", 0)));
@@ -285,10 +288,20 @@ LaunchPlan PlanAndLaunchOe(sbnb_engine* e, OeParams p, bool launch, int chunks_o
   return plan;
 }
 
-template <int C, int K, bool GRAD, bool SUBST, bool AMBIG, bool INVAR>
+template <int C, int K, bool GRAD, bool SUBST, bool AMBIG, bool INVAR, bool SITES = false>
 LaunchPlan DispatchRescale(sbnb_engine* e, const OeParams& p, bool rescale, bool launch, int chunks_override) {
-  return rescale ? PlanAndLaunchOe<C, K, GRAD, true, SUBST, AMBIG, INVAR>(e, p, launch, chunks_override)
-                 : PlanAndLaunchOe<C, K, GRAD, false, SUBST, AMBIG, INVAR>(e, p, launch, chunks_override);
+  return rescale ? PlanAndLaunchOe<C, K, GRAD, true, SUBST, AMBIG, INVAR, SITES>(e, p, launch, chunks_override)
+                 : PlanAndLaunchOe<C, K, GRAD, false, SUBST, AMBIG, INVAR, SITES>(e, p, launch, chunks_override);
+}
+
+// A log-likelihood run with p.site_logl set runs the walks that also store the log site
+// likelihoods; every other run the walks without the store (a compile-time variant: their code
+// is unchanged).  The two have the same tiling, so their log-likelihoods are bitwise equal.
+template <int C, int K, bool AMBIG, bool INVAR>
+LaunchPlan DispatchSitesOe(sbnb_engine* e, const OeParams& p, bool rescale, bool launch, int chunks_override) {
+  return p.site_logl != nullptr
+             ? DispatchRescale<C, K, false, false, AMBIG, INVAR, true>(e, p, rescale, launch, chunks_override)
+             : DispatchRescale<C, K, false, false, AMBIG, INVAR>(e, p, rescale, launch, chunks_override);
 }
 
 // K_GRAD / K_LOGL patterns per thread for the gradient / logL-only walk; a gradient walk
@@ -299,7 +312,7 @@ LaunchPlan DispatchModesOe(sbnb_engine* e, const OeParams& p, bool grad, bool re
   if (grad && p.subst_partial != nullptr)
     return DispatchRescale<C, K_GRAD, true, true, AMBIG, INVAR>(e, p, rescale, launch, chunks_override);
   return grad ? DispatchRescale<C, K_GRAD, true, false, AMBIG, INVAR>(e, p, rescale, launch, chunks_override)
-              : DispatchRescale<C, K_LOGL, false, false, AMBIG, INVAR>(e, p, rescale, launch, chunks_override);
+              : DispatchSitesOe<C, K_LOGL, AMBIG, INVAR>(e, p, rescale, launch, chunks_override);
 }
 
 // A site model with invariable sites (+I) runs the walks with the invariant class at the root
@@ -591,7 +604,7 @@ void WaitForStaging(sbnb_engine* e) {
 }
 
 BatchPtr Stage(sbnb_engine* e, const sbnb_tree_batch* trees, const double* params, bool rooted,
-               bool with_fd, bool slide_root, bool with_subst = false) {
+               bool with_fd, bool slide_root, bool with_subst = false, bool with_sites = false) {
   NvtxRange range("sbnb stage");
   CheckTrees(e, trees, rooted);
   const ModelSpec& spec = e->spec;
@@ -613,6 +626,7 @@ BatchPtr Stage(sbnb_engine* e, const sbnb_tree_batch* trees, const double* param
   batch->fd_coords = fd_evals / 2;
   batch->with_subst = with_subst;
   batch->invariant = spec.invariant;
+  batch->with_sites = with_sites;
   batch->site_width = spec.SiteGradientSize();
   batch->vtree_count = T * (1 + fd_evals);
   if (T == 0) return batch;
@@ -763,6 +777,7 @@ BatchPtr Stage(sbnb_engine* e, const sbnb_tree_batch* trees, const double* param
   batch->results.Reserve(batch->vtree_count + 2 * static_cast<size_t>(T) * N +
                          static_cast<size_t>(T) * (kOeSubstSums + kOeInvariantSums) + (batch->rooted_finish ? static_cast<size_t>(T) * batch->RootedWidth() : 0));
   if (batch->rooted_finish) batch->rooted_scratch.Reserve(static_cast<size_t>(T) * 5 * (n - 1));
+  if (with_sites) batch->site_logl.Reserve(static_cast<size_t>(T) * batch->patterns);
   return batch;
 }
 
@@ -879,6 +894,13 @@ void Run(sbnb_engine* e, sbnb_batch* b, int mode, bool rescaling, bool timed = t
   p.subst_partial = subst ? b->subst_partial.get() : nullptr;
   const bool inv = grad && b->invariant;
   p.inv_partial = inv ? b->inv_partial.get() : nullptr;
+  if (!grad && b->with_sites) {
+    // (planned above without it: the walk that stores the sites runs the same tiling; a
+    //  log-likelihood run has no finite-difference evaluations, so only the T trees write)
+    Require(e->range_end - e->range_begin == b->patterns,
+            "The pattern range has changed since the batch was staged for site log-likelihoods.");
+    p.site_logl = b->site_logl.get();
+  }
 
   // Base trees: matrices, then the logL or gradient sweep.
   b->operand_stride = grad ? b->full_doubles : b->post_doubles;
@@ -993,10 +1015,27 @@ void Unpack(const sbnb_engine* e, const sbnb_batch* b, const double* landed, dou
   }
 }
 
+// Doubles of a batch's site matrix, [T][patterns].
+size_t SiteCount(const sbnb_batch* b) { return static_cast<size_t>(b->tree_count) * b->patterns; }
+
+// The landing area of one fetch: `count` doubles of the result array, then (sites) the site matrix.
+double* Land(sbnb_engine* e, size_t count, size_t site_count, double** landed_sites) {
+  e->landing.Reset((count + site_count) * sizeof(double) + 256);
+  double* landed = e->landing.Take<double>(count);
+  *landed_sites = site_count ? e->landing.Take<double>(site_count) : nullptr;
+  return landed;
+}
+
 void Fetch(sbnb_engine* e, sbnb_batch* b, double* logl, double* grad, double* rgrad, double* subst = nullptr,
-           double* rooted = nullptr, double* inv = nullptr) {
+           double* rooted = nullptr, double* inv = nullptr, double* sites = nullptr) {
   NvtxRange range("sbnb fetch");
   SBNB_CUDA(cudaSetDevice(e->device));
+  if (sites) {
+    Require(b->with_sites, "No site log-likelihoods: the batch was not staged with SBNB_STAGE_SITE_LOG_LIKELIHOODS.");
+    Require(b->last_mode >= 0, "No site log-likelihoods: the batch has not been run yet.");
+    Require(b->last_mode == SBNB_MODE_LOG_LIKELIHOOD,
+            "No site log-likelihoods: the last run was a gradient run (log-likelihood runs write them).");
+  }
   Require(b->last_mode >= 0, "sbnb_batch_fetch called before sbnb_batch_run.");
   const bool was_grad = (b->last_mode == SBNB_MODE_BRANCH_GRADIENT);
   Require(was_grad || (!grad && !rgrad), "No gradient available: the last run was a log-likelihood run.");
@@ -1011,12 +1050,16 @@ void Fetch(sbnb_engine* e, sbnb_batch* b, double* logl, double* grad, double* rg
   if (rooted) Require(was_grad && b->rooted_finish, "No finished rooted gradients: the batch carries no time-tree fields.");
   const size_t count =
       FetchCount(e, b, grad != nullptr, rgrad != nullptr, subst != nullptr, rooted != nullptr, inv != nullptr);
-  e->landing.Reset(count * sizeof(double));
-  double* landed = e->landing.Take<double>(count);
+  const size_t site_count = sites ? SiteCount(b) : 0;
+  double* landed_sites = nullptr;
+  double* landed = Land(e, count, site_count, &landed_sites);
   SBNB_CUDA(cudaMemcpyAsync(landed, b->results.get(), count * sizeof(double), cudaMemcpyDeviceToHost, s));
-  e->d2h_bytes += count * sizeof(double);
+  if (sites)
+    SBNB_CUDA(cudaMemcpyAsync(landed_sites, b->site_logl.get(), site_count * sizeof(double), cudaMemcpyDeviceToHost, s));
+  e->d2h_bytes += (count + site_count) * sizeof(double);
   SBNB_CUDA(cudaStreamSynchronize(s));
   Unpack(e, b, landed, logl, grad, rgrad, subst, rooted, inv);
+  if (sites) std::copy(landed_sites, landed_sites + site_count, sites);
 }
 
 // Run + Fetch of the one-call entry points.  Once the same topology set has come in
@@ -1025,12 +1068,14 @@ void Fetch(sbnb_engine* e, sbnb_batch* b, double* logl, double* grad, double* rg
 // 4-6 launches, 2 event records and a copy (the small-problem regime of
 // BASELINE.json configs[0..1], where a call is tens of microseconds).
 void RunAndFetch(sbnb_engine* e, sbnb_batch* b, int mode, bool rescaling, double* logl, double* grad,
-                 double* rgrad, double* subst = nullptr, double* rooted = nullptr, double* inv = nullptr) {
+                 double* rgrad, double* subst = nullptr, double* rooted = nullptr, double* inv = nullptr,
+                 double* sites = nullptr) {
   static const bool graphs_enabled = EnvInt("SBNB_GRAPHS", 1) != 0;
-  sbnb_batch::Graph& graph = b->graphs[mode == SBNB_MODE_BRANCH_GRADIENT ? 1 : 0][rescaling ? 1 : 0];
+  sbnb_batch::Graph& graph =
+      b->graphs[mode == SBNB_MODE_BRANCH_GRADIENT ? 1 : (b->with_sites ? 2 : 0)][rescaling ? 1 : 0];
   if (!graphs_enabled || b->tree_count == 0 || b->cache_hits < 1 || !graph.warm) {
     Run(e, b, mode, rescaling);
-    Fetch(e, b, logl, grad, rgrad, subst, rooted, inv);
+    Fetch(e, b, logl, grad, rgrad, subst, rooted, inv, sites);
     graph.warm = b->cache_hits >= 1;  // (an eager run on cached programs: the next one may be captured)
     return;
   }
@@ -1039,8 +1084,9 @@ void RunAndFetch(sbnb_engine* e, sbnb_batch* b, int mode, bool rescaling, double
   b->last_mode = mode;
   const size_t count =
       FetchCount(e, b, grad != nullptr, rgrad != nullptr, subst != nullptr, rooted != nullptr, inv != nullptr);
-  e->landing.Reset(count * sizeof(double));
-  double* landed = e->landing.Take<double>(count);
+  const size_t site_count = sites ? SiteCount(b) : 0;
+  double* landed_sites = nullptr;
+  double* landed = Land(e, count, site_count, &landed_sites);
   auto signature = [&] {
     return std::vector<uintptr_t>{
         reinterpret_cast<uintptr_t>(b->input.get()),        reinterpret_cast<uintptr_t>(b->operands.get()),
@@ -1053,7 +1099,9 @@ void RunAndFetch(sbnb_engine* e, sbnb_batch* b, int mode, bool rescaling, double
         static_cast<uintptr_t>(count),                      static_cast<uintptr_t>(b->vtree_count),
         static_cast<uintptr_t>(b->with_subst),              static_cast<uintptr_t>(e->range_end - e->range_begin),
         static_cast<uintptr_t>(b->slots),                   reinterpret_cast<uintptr_t>(b->rooted_scratch.get()),
-        reinterpret_cast<uintptr_t>(b->inv_partial.get()),  reinterpret_cast<uintptr_t>(e->invariant_masks.get())};
+        reinterpret_cast<uintptr_t>(b->inv_partial.get()),  reinterpret_cast<uintptr_t>(e->invariant_masks.get()),
+        reinterpret_cast<uintptr_t>(b->site_logl.get()),    reinterpret_cast<uintptr_t>(landed_sites),
+        static_cast<uintptr_t>(site_count)};
   };
   if (graph.exec == nullptr || graph.signature != signature()) {
     if (graph.exec) {
@@ -1068,6 +1116,9 @@ void RunAndFetch(sbnb_engine* e, sbnb_batch* b, int mode, bool rescaling, double
     try {
       Run(e, b, mode, rescaling, /*timed=*/false);
       SBNB_CUDA(cudaMemcpyAsync(landed, b->results.get(), count * sizeof(double), cudaMemcpyDeviceToHost, s));
+      if (sites)
+        SBNB_CUDA(cudaMemcpyAsync(landed_sites, b->site_logl.get(), site_count * sizeof(double),
+                                  cudaMemcpyDeviceToHost, s));
     } catch (...) {
       cudaStreamEndCapture(s, &recorded);
       if (recorded) cudaGraphDestroy(recorded);
@@ -1083,9 +1134,10 @@ void RunAndFetch(sbnb_engine* e, sbnb_batch* b, int mode, bool rescaling, double
   }
   SBNB_CUDA(cudaGraphLaunch(graph.exec, s));
   e->launch_count += graph.kernels;
-  e->d2h_bytes += count * sizeof(double);
+  e->d2h_bytes += (count + site_count) * sizeof(double);
   SBNB_CUDA(cudaStreamSynchronize(s));
   Unpack(e, b, landed, logl, grad, rgrad, subst, rooted, inv);
+  if (sites) std::copy(landed_sites, landed_sites + site_count, sites);
 }
 
 RootedView ViewOf(const sbnb_tree_batch* trees, int t, int n) {
@@ -1179,13 +1231,15 @@ std::unique_ptr<sbnb_engine> CreateEngine(const char* substitution, const char* 
   return engine;
 }
 
-// The one-call forms of Engine's five methods.
+// The one-call forms of Engine's five methods.  `sites` (NULL or [T][patterns of the engine's
+// range]) also receives every pattern's log site likelihood, without the Jacobian.
 void LogLikelihoods(sbnb_engine* e, const sbnb_tree_batch* trees, const double* params,
-                    bool rescaling, bool rooted_semantics, bool add_jacobian, double* out) {
+                    bool rescaling, bool rooted_semantics, bool add_jacobian, double* out, double* sites = nullptr) {
   Require(trees != nullptr, "NULL tree batch.");
   Require(out != nullptr || trees->tree_count == 0, "NULL output.");
-  auto batch = Stage(e, trees, params, rooted_semantics, false, /*slide_root=*/false);
-  RunAndFetch(e, batch.get(), SBNB_MODE_LOG_LIKELIHOOD, rescaling, out, nullptr, nullptr);
+  auto batch = Stage(e, trees, params, rooted_semantics, false, /*slide_root=*/false, false, sites != nullptr);
+  RunAndFetch(e, batch.get(), SBNB_MODE_LOG_LIKELIHOOD, rescaling, out, nullptr, nullptr, nullptr, nullptr, nullptr,
+              sites);
   if (add_jacobian) {
     Require(trees->tree_count == 0 || (trees->node_heights && trees->node_bounds),
             "Rooted log likelihoods need node_heights and node_bounds.");
@@ -1377,13 +1431,13 @@ sbnb_tree_batch SliceTrees(const sbnb_tree_batch* trees, int n, int begin, int e
 // Returns child 0's batch (results complete once its stream has been synchronised).
 std::vector<BatchPtr> RunOverPatternShards(sbnb_engine* group, const sbnb_tree_batch* trees, const double* params,
                                            bool rooted, bool with_fd, bool slide_root, int mode, bool rescaling,
-                                           bool with_subst = false) {
+                                           bool with_subst = false, bool with_sites = false) {
   const int G = static_cast<int>(group->children.size());
   std::vector<BatchPtr> batches;
   for (int g = 0; g < G; g++) batches.emplace_back(nullptr, BatchRecycler{group->children[g]});
   std::vector<cudaEvent_t> done(G, nullptr);
   ParallelOverChildren(group, [&](int g, sbnb_engine* child) {
-    batches[g] = Stage(child, trees, params, rooted, with_fd, slide_root, with_subst);
+    batches[g] = Stage(child, trees, params, rooted, with_fd, slide_root, with_subst, with_sites);
     Run(child, batches[g].get(), mode, rescaling);
     if (g > 0) {
       SBNB_CUDA(cudaEventCreateWithFlags(&done[g], cudaEventDisableTiming));
@@ -1440,11 +1494,12 @@ std::vector<BatchPtr> RunOverPatternShards(sbnb_engine* group, const sbnb_tree_b
 }
 
 void GroupLogLikelihoods(sbnb_engine* group, const sbnb_tree_batch* trees, const double* params, bool rescaling,
-                         bool rooted_semantics, bool add_jacobian, double* out) {
+                         bool rooted_semantics, bool add_jacobian, double* out, double* sites = nullptr) {
   Require(trees != nullptr, "NULL tree batch.");
   Require(out != nullptr || trees->tree_count == 0, "NULL output.");
   const int G = static_cast<int>(group->children.size()), T = trees->tree_count, n = group->taxon_count;
   const int K = group->spec.param_count;
+  const int64_t P = group->pattern_count;
   if (group->shard_axis == SBNB_SHARD_TREES) {
     ParallelOverChildren(group, [&](int g, sbnb_engine* child) {
       const int begin = static_cast<int>(static_cast<int64_t>(T) * g / G);
@@ -1452,13 +1507,23 @@ void GroupLogLikelihoods(sbnb_engine* group, const sbnb_tree_batch* trees, const
       if (begin == end) return;
       const sbnb_tree_batch slice = SliceTrees(trees, n, begin, end);
       LogLikelihoods(child, &slice, params ? params + static_cast<size_t>(begin) * K : nullptr, rescaling,
-                     rooted_semantics, add_jacobian, out + begin);
+                     rooted_semantics, add_jacobian, out + begin, sites ? sites + begin * P : nullptr);
     });
     return;
   }
   auto batches = RunOverPatternShards(group, trees, params, rooted_semantics, false, false,
-                                      SBNB_MODE_LOG_LIKELIHOOD, rescaling);
+                                      SBNB_MODE_LOG_LIKELIHOOD, rescaling, false, sites != nullptr);
   Fetch(group->children[0], batches[0].get(), out, nullptr, nullptr);
+  if (sites && T > 0) {
+    // Nothing to add: every child's [T][its range] block goes to its columns of [T][P].
+    ParallelOverChildren(group, [&](int g, sbnb_engine* child) {
+      const int64_t range = child->range_end - child->range_begin;
+      std::vector<double> block(static_cast<size_t>(T) * range);
+      Fetch(child, batches[g].get(), nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, block.data());
+      for (int t = 0; t < T; t++)
+        std::copy(block.begin() + t * range, block.begin() + (t + 1) * range, sites + t * P + child->range_begin);
+    });
+  }
   if (add_jacobian) {
     Require(T == 0 || (trees->node_heights && trees->node_bounds),
             "Rooted log likelihoods need node_heights and node_bounds.");
@@ -1633,7 +1698,7 @@ int sbnb_log_likelihoods_unrooted(sbnb_engine* engine, const sbnb_tree_batch* tr
                                   const double* params, int32_t rescaling, double* out) {
   return Guard([&] {
     Require(engine != nullptr, "NULL engine.");
-    (IsGroup(engine) ? GroupLogLikelihoods : LogLikelihoods)(engine, trees, params, rescaling != 0, false, false, out);
+    (IsGroup(engine) ? GroupLogLikelihoods : LogLikelihoods)(engine, trees, params, rescaling != 0, false, false, out, nullptr);
   });
 }
 
@@ -1641,8 +1706,35 @@ int sbnb_log_likelihoods_rooted(sbnb_engine* engine, const sbnb_tree_batch* tree
                                 const double* params, int32_t rescaling, double* out) {
   return Guard([&] {
     Require(engine != nullptr, "NULL engine.");
-    (IsGroup(engine) ? GroupLogLikelihoods : LogLikelihoods)(engine, trees, params, rescaling != 0, true, true, out);
+    (IsGroup(engine) ? GroupLogLikelihoods : LogLikelihoods)(engine, trees, params, rescaling != 0, true, true, out, nullptr);
   });
+}
+
+// sbnb_site_log_likelihoods_*: the log-likelihoods (rooted: with the Jacobian) and the [T][P] site
+// matrix (without it) of one log-likelihood run.
+static int SiteLogLikelihoods(sbnb_engine* engine, const sbnb_tree_batch* trees, const double* params,
+                              int32_t rescaling, bool rooted, double* out_log_likelihoods, double* out_site) {
+  return Guard([&] {
+    Require(engine != nullptr, "NULL engine.");
+    Require(trees != nullptr, "NULL tree batch.");
+    Require(out_site != nullptr || trees->tree_count == 0, "NULL site log-likelihood output.");
+    std::vector<double> logl(out_log_likelihoods ? 0 : std::max(trees->tree_count, 0));
+    double* out = out_log_likelihoods ? out_log_likelihoods : logl.data();
+    if (IsGroup(engine))
+      GroupLogLikelihoods(engine, trees, params, rescaling != 0, rooted, rooted, out, out_site);
+    else
+      LogLikelihoods(engine, trees, params, rescaling != 0, rooted, rooted, out, out_site);
+  });
+}
+
+int sbnb_site_log_likelihoods_unrooted(sbnb_engine* engine, const sbnb_tree_batch* trees, const double* params,
+                                       int32_t rescaling, double* out_log_likelihoods, double* out_site) {
+  return SiteLogLikelihoods(engine, trees, params, rescaling, false, out_log_likelihoods, out_site);
+}
+
+int sbnb_site_log_likelihoods_rooted(sbnb_engine* engine, const sbnb_tree_batch* trees, const double* params,
+                                     int32_t rescaling, double* out_log_likelihoods, double* out_site) {
+  return SiteLogLikelihoods(engine, trees, params, rescaling, true, out_log_likelihoods, out_site);
 }
 
 int sbnb_unrooted_log_likelihoods_of_rooted(sbnb_engine* engine, const sbnb_tree_batch* trees,
@@ -1652,7 +1744,7 @@ int sbnb_unrooted_log_likelihoods_of_rooted(sbnb_engine* engine, const sbnb_tree
     // fat_beagle.cpp:78-80: plain branch lengths, no rates, no Jacobian.
     Require(trees && trees->node_count == 2 * engine->taxon_count - 1,
             "Rooted trees must be bifurcating: node_count must be 2n-1.");
-    (IsGroup(engine) ? GroupLogLikelihoods : LogLikelihoods)(engine, trees, params, rescaling != 0, false, false, out);
+    (IsGroup(engine) ? GroupLogLikelihoods : LogLikelihoods)(engine, trees, params, rescaling != 0, false, false, out, nullptr);
   });
 }
 
@@ -1726,7 +1818,8 @@ int sbnb_batch_stage(sbnb_engine* engine, const sbnb_tree_batch* trees, const do
             "A batch is staged for one substitution-gradient method.");
     *out = Stage(engine, trees, params, (stage_flags & SBNB_STAGE_ROOTED) != 0,
                  (stage_flags & SBNB_STAGE_SUBSTITUTION_FD) != 0, /*slide_root=*/true,
-                 (stage_flags & SBNB_STAGE_SUBSTITUTION_ANALYTIC) != 0 && engine->spec.SubstitutionGradientSize() > 0)
+                 (stage_flags & SBNB_STAGE_SUBSTITUTION_ANALYTIC) != 0 && engine->spec.SubstitutionGradientSize() > 0,
+                 (stage_flags & SBNB_STAGE_SITE_LOG_LIKELIHOODS) != 0)
                .release();
   });
 }
@@ -1753,6 +1846,14 @@ int sbnb_batch_fetch_substitution_sums(sbnb_engine* engine, sbnb_batch* batch, d
     Require(engine && batch && sums, "NULL argument.");
     RequireSingleDevice(engine);
     Fetch(engine, batch, nullptr, nullptr, nullptr, sums);
+  });
+}
+
+int sbnb_batch_fetch_site_log_likelihoods(sbnb_engine* engine, sbnb_batch* batch, double* out) {
+  return Guard([&] {
+    Require(engine && batch && out, "NULL argument.");
+    RequireSingleDevice(engine);
+    Fetch(engine, batch, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, out);
   });
 }
 

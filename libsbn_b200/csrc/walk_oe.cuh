@@ -106,6 +106,7 @@ struct OeParams {
   double* subst_partial;   // [vtree][chunk][warp][kOeSubstSums]        (analytic substitution gradient)
   const uint8_t* invariant_masks;  // [tip_pitch] the states every tip allows, per pattern (+I; 0 = padding)
   double* inv_partial;     // [vtree][chunk][warp][kOeInvariantSums]    (+I gradient runs)
+  double* site_logl;       // [vtree][pattern - pattern_begin] log site likelihoods (SITES walks)
 };
 
 // ---------------------------------------------------------------------------
@@ -651,9 +652,13 @@ __device__ __forceinline__ InvariantSiteTerms InvariantSite(double log_l, double
   return t;
 }
 
-template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false, bool AMBIG = false, bool INVAR = false>
+// SITES (logL-only walks): the root op also stores every pattern's log site likelihood -- the
+// term it adds into logL with the pattern's weight -- into p.site_logl.
+template <int C, int K, bool GRAD, bool RESCALE, bool SUBST = false, bool AMBIG = false, bool INVAR = false,
+          bool SITES = false>
 __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWalkOeKernel(const OeParams p) {
   static_assert(GRAD || !SUBST, "the substitution gradient rides on the pre-order pass");
+  static_assert(!(GRAD && SITES), "site log-likelihoods come from log-likelihood runs");
   static_assert((C & (C - 1)) == 0 && C >= 1 && C <= 32, "lanes per pattern must be a power of two");
   static_assert(OeTilePatterns(C, K) % 16 == 0, "tiles must start on 16-byte boundaries of the tip rows");
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -1013,6 +1018,13 @@ __global__ void __launch_bounds__(kThreads, OeMinBlocks(K, GRAD, SUBST)) TreeWal
                   if (mask >> s & 1u) invariant += freqs[s];
                 inv = InvariantSite(log_site, site, RESCALE ? cur_exp[j] : 0, pinv, invariant);
                 log_site = inv.log_lik;
+              }
+              if constexpr (SITES) {
+                // the same lane stores it, whatever the weight; the padding is never written
+                const int64_t pattern = pat0 + pidx * K + j;
+                if (cat == 0 && pattern < p.pattern_end)
+                  p.site_logl[static_cast<int64_t>(vt) * (p.pattern_end - p.pattern_begin) + (pattern - p.pattern_begin)] =
+                      log_site;
               }
               // one lane per pattern carries the term
               logl_acc = fma(w[j], (w[j] != 0.0 && cat == 0) ? log_site : 0.0, logl_acc);

@@ -92,11 +92,12 @@ class TreeBatch:
 class StagedBatch:
     """A tree collection staged in device memory (sbnb_batch)."""
 
-    def __init__(self, engine, handle, tree_count, node_count):
+    def __init__(self, engine, handle, tree_count, node_count, pattern_count=None):
         self._engine = engine
         self._handle = handle
         self.tree_count = tree_count
         self.node_count = node_count  # 2n-1
+        self.pattern_count = pattern_count  # width of the engine's pattern range when staged
 
     def run(self, mode=_capi.MODE_LOG_LIKELIHOOD, rescaling=False):
         """Enqueue one pass on the engine's stream (no copies, no sync)."""
@@ -118,6 +119,14 @@ class StagedBatch:
         _capi.check(_capi.load().sbnb_batch_fetch_substitution_sums(self._engine._handle, self._handle,
                                                                     _capi.as_double_ptr(sums)))
         return sums
+
+    def fetch_site_log_likelihoods(self):
+        """[T][P] log site likelihoods of the last (log-likelihood) run of a batch staged with
+        site_log_likelihoods=True; P = the engine's pattern range when staged."""
+        sites = np.empty((self.tree_count, self.pattern_count))
+        _capi.check(_capi.load().sbnb_batch_fetch_site_log_likelihoods(self._engine._handle, self._handle,
+                                                                       _capi.as_double_ptr(sites)))
+        return sites
 
     def fetch_invariant_sums(self):
         """[T][5] sums of the invariant class (D, E_A..E_T) of the last gradient run of a +I model."""
@@ -160,6 +169,7 @@ class Engine:
         self.specification = specification
         self.tip_encoding = tip_encoding
         self.taxon_count, self.pattern_count = patterns.shape
+        self.pattern_range = (0, self.pattern_count)
         handle = ctypes.c_void_p()
         common = (specification.substitution.encode(), specification.site.encode(),
                   specification.clock.encode(), self.taxon_count, self.pattern_count,
@@ -246,6 +256,22 @@ class Engine:
                        _capi.as_double_ptr(out)))
         return out
 
+    def site_log_likelihoods(self, trees, params=None, rescaling=False, rooted=False):
+        """(logL [T], site log-likelihoods [T][P]) of one log-likelihood run: site[t, k] is the
+        log likelihood of pattern k of the engine's pattern range under tree t, unweighted, so
+        that site @ weights = logL (rooted: logL minus the log-det Jacobian, which logL includes).
+        Weight-0 patterns get their values too.  A device group returns all pattern_count columns."""
+        lib = _capi.load()
+        params = self._params(params, trees.tree_count)
+        width = self.pattern_count if self.device_count > 1 else self.pattern_range[1] - self.pattern_range[0]
+        logl = np.empty(trees.tree_count, dtype=np.float64)
+        sites = np.empty((trees.tree_count, width), dtype=np.float64)
+        fn = lib.sbnb_site_log_likelihoods_rooted if rooted else lib.sbnb_site_log_likelihoods_unrooted
+        struct = trees.as_struct()
+        _capi.check(fn(self._handle, ctypes.byref(struct), _capi.as_double_ptr(params), int(rescaling),
+                       _capi.as_double_ptr(logl), _capi.as_double_ptr(sites)))
+        return logl, sites
+
     def unrooted_log_likelihoods(self, trees, params=None, rescaling=False):
         """Engine::UnrootedLogLikelihoods(RootedTreeCollection)."""
         params = self._params(params, trees.tree_count)
@@ -288,18 +314,24 @@ class Engine:
         return results
 
     # -- staged form -------------------------------------------------------------
-    def stage(self, trees, params=None, rooted=False, substitution_fd=False, substitution_analytic=False):
+    def stage(self, trees, params=None, rooted=False, substitution_fd=False, substitution_analytic=False,
+              site_log_likelihoods=False):
+        """site_log_likelihoods: log-likelihood runs also write the [T][P] site matrix
+        (StagedBatch.fetch_site_log_likelihoods), T x P doubles of device memory."""
         params = self._params(params, trees.tree_count)
         flags = (_capi.STAGE_ROOTED if rooted else 0) | (_capi.STAGE_SUBSTITUTION_FD if substitution_fd else 0) | \
-            (_capi.STAGE_SUBSTITUTION_ANALYTIC if substitution_analytic else 0)
+            (_capi.STAGE_SUBSTITUTION_ANALYTIC if substitution_analytic else 0) | \
+            (_capi.STAGE_SITE_LOG_LIKELIHOODS if site_log_likelihoods else 0)
         handle = ctypes.c_void_p()
         struct = trees.as_struct()
         _capi.check(_capi.load().sbnb_batch_stage(self._handle, ctypes.byref(struct),
                                                   _capi.as_double_ptr(params), flags, ctypes.byref(handle)))
-        return StagedBatch(self, handle, trees.tree_count, 2 * self.taxon_count - 1)
+        return StagedBatch(self, handle, trees.tree_count, 2 * self.taxon_count - 1,
+                           self.pattern_range[1] - self.pattern_range[0])
 
     def set_pattern_range(self, begin, end):
         _capi.check(_capi.load().sbnb_engine_set_pattern_range(self._handle, begin, end))
+        self.pattern_range = (begin, end)
 
     @property
     def stream(self):

@@ -117,6 +117,13 @@ class TreeShardedEngine:
         local = self.engine.log_likelihoods(local_trees, local_params, rescaling, rooted)
         return all_gather_rows(local[:, None], trees.tree_count)[:, 0]
 
+    def site_log_likelihoods(self, trees, params=None, rescaling=False, rooted=False):
+        """(logL [T], site log-likelihoods [T][P]) on every rank: the local rows, all-gathered."""
+        _, _, local_trees, local_params = self.local_slice(trees, params)
+        logl, sites = self.engine.site_log_likelihoods(local_trees, local_params, rescaling, rooted)
+        rows = all_gather_rows(np.concatenate([logl[:, None], sites], axis=1), trees.tree_count)
+        return rows[:, 0].copy(), np.ascontiguousarray(rows[:, 1:])
+
     def gradients(self, trees, params=None, rescaling=False, rooted=False, substitution_gradient=True):
         _, _, local_trees, local_params = self.local_slice(trees, params)
         local = self.engine.gradients(local_trees, local_params, rescaling, rooted, substitution_gradient)
@@ -276,6 +283,7 @@ class PatternShardedEngine:
         self.rank, self.world, self.backend = _world()
         self.specification = specification
         self.engine = Engine(specification, patterns, weights, device, tip_encoding=tip_encoding)
+        self.presharded = presharded
         if presharded:
             self.begin, self.end = 0, self.engine.pattern_count
         else:
@@ -332,6 +340,21 @@ class PatternShardedEngine:
         if rooted:
             finish_log_likelihoods_rooted(self.engine.taxon_count, trees, logl)
         return logl
+
+    def site_log_likelihoods(self, trees, params=None, rescaling=False, rooted=False):
+        """(logL [T], site log-likelihoods [T][pattern_count]) on every rank: the log-likelihoods
+        sum-all-reduced, this rank's [T][P_r] columns all-gathered (transposed: the ranks' rows are
+        their pattern ranges, which follow shard_range)."""
+        if self.presharded:
+            raise RuntimeError("site_log_likelihoods needs the whole alignment on every rank (presharded=False).")
+        staged = self.engine.stage(trees, params, rooted=rooted, site_log_likelihoods=True)
+        staged.run(_capi.MODE_LOG_LIKELIHOOD, rescaling)
+        logl = self._reduce(staged, 1)
+        local = staged.fetch_site_log_likelihoods()
+        staged.close()
+        if rooted:
+            finish_log_likelihoods_rooted(self.engine.taxon_count, trees, logl)
+        return logl, np.ascontiguousarray(all_gather_rows(np.ascontiguousarray(local.T), self.engine.pattern_count).T)
 
     def gradients(self, trees, params=None, rescaling=False, rooted=False, substitution_gradient=True):
         wanted = substitution_gradient and self.specification.substitution in ("GTR", "HKY")
